@@ -12,11 +12,16 @@ configs[2] BIWI 128 clips x 6 s over N GPUs and configs[3] MEAD 256 clips x 8 s 
 anchor of the strong-scaling curve). `microbench` (N = 1) is configs[4]: EVQ-VAE quantise / decode and HuBERT encode at
 1024 clips x 10 s with a roofline per stage.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes the vertices the last timed job of the headline workload returned to DIR/vertices.npy (see
+dump_vertices); inputs, weights and sampling noise are seeded, so two builds run with the same arguments can be compared
+output for output.
 
 --impl reference times the REAL reference modules (copied unmodified by __graft_entry__.build() into the git-ignored
 oracle/_ref, run by oracle/ref_runner.py in a subprocess) on the host cores; without oracle/_ref it falls back to the
-oracle port and says so (`cpu_baseline.kind`).
+oracle port and says so (`cpu_baseline.kind`). build() fills oracle/_ref only when FDM_B200_REFERENCE_DIR names a
+checkout of the reference, so set it there to time the reference itself.
 """
 import argparse
 import json
@@ -55,7 +60,11 @@ def parse():
     ap.add_argument("--named", default="auto", choices=["auto", "none"], help="also run BASELINE configs[2] / configs[3], strong-sharded")
     ap.add_argument("--microbench", default="auto", choices=["auto", "none"], help="also run BASELINE configs[4] (N = 1 only)")
     ap.add_argument("--gather-chunks", type=int, default=0, help="decode / all-gather chunks (0 = automatic)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the vertices of the last timed job to DIR/vertices.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload_config(args, world):
@@ -118,6 +127,31 @@ def synthetic_audio(n_clips, n_samples, clip0):
         a = torch.randn(n_samples, generator=g)
         out[i] = (a - a.mean()) / a.std()
     return out
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_vertices(out_dir, verts):
+    """verts (clips, frames, V * 3) -> out_dir/vertices.npy, float32 (c, frames, n, 3): all of it when it fits in
+    DUMP_BYTES, else a fixed, seeded subset of n vertices, the same for every clip and frame (the headline workload's
+    64 clips x 198 frames keep 420 of the 5023 vertices), and of c clips too when one vertex of every clip would not fit."""
+    import numpy as np
+    clips, frames, v3 = verts.shape
+    budget = DUMP_BYTES - 1024  # room for the .npy header
+    track = frames * 3 * 4  # bytes of one vertex over one clip's frames
+    if track > budget:
+        raise ValueError(f"--dump-outputs: one vertex of one clip over {frames} frames exceeds {DUMP_BYTES} bytes")
+    g = torch.Generator().manual_seed(0)
+    v = verts.view(clips, frames, v3 // 3, 3)
+    c = min(clips, budget // track)
+    if c < clips:
+        v = v[torch.randperm(clips, generator=g)[:c].sort().values.to(v.device)]
+    n = min(v3 // 3, budget // (c * track))
+    if n < v3 // 3:
+        v = v[:, :, torch.randperm(v3 // 3, generator=g)[:n].sort().values.to(v.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "vertices.npy"), v.float().cpu().numpy())
 
 
 class ClockSampler:
@@ -389,7 +423,7 @@ class Workload:
         self.gather.run(lambda k0, k1, dst: self.ae.decode(zq, out=dst, clips=(k0, k1)), self.gathered, time_it=time_gather)
         return self.gathered[self.rank]
 
-    def measure(self, steps, warmup, e2e=True):
+    def measure(self, steps, warmup, e2e=True, dump_dir=None):
         from fdm_b200 import lib
         world, dev = self.world, self.dev
 
@@ -417,6 +451,8 @@ class Workload:
         ms_dev = e0.elapsed_time(e1)
         den_ms = [s.step_ms() for s in samplers]
         gather_ms = self.gather.exposed_gather_ms()
+        if dump_dir:  # before the end-to-end leg reuses the buffer; after the all-gather it holds every rank's clips
+            dump_vertices(dump_dir, self.gathered.flatten(0, 1))
         ms_e2e = None
         if e2e:
             self.verts_host = torch.empty(self.B, self.T, self.V3).pin_memory()
@@ -627,7 +663,7 @@ def main():
     if rank == 0:
         sampler.start()
     wl = Workload(args.preset, args.clips, args.seconds, args, rank, world, dev)
-    m = wl.measure(args.steps, args.warmup, e2e=True)
+    m = wl.measure(args.steps, args.warmup, e2e=True, dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
     roof, extra, flops = (None, {}, None)
     if rank == 0:

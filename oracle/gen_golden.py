@@ -1,12 +1,12 @@
-"""Generate tests/golden/*.npz|json by running the REAL reference (TEST INFRASTRUCTURE; build container only).
+"""Generate tests/golden/*.npz|json by running the REAL reference (TEST INFRASTRUCTURE; needs a reference checkout).
 
-Imports the reference's own modules from /root/reference with the harness shims of SURVEY.md §8(c), gives them
-the deterministic weights of oracle/weights.py, and records (a) their state_dict layout, (b) their outputs on
-seeded inputs. While doing so it checks the oracle restatement (oracle/reference_ops.py) against the reference
-and refuses to write fixtures if they disagree. /root/reference does not exist on the GPU box: the committed
-fixtures are what travels.
+Imports the reference's own modules from the checkout FDM_B200_REFERENCE_DIR names, with the harness shims of
+SURVEY.md §8(c), gives them the deterministic weights of oracle/weights.py, and records (a) their state_dict layout,
+(b) their outputs on seeded inputs. While doing so it checks the oracle restatement (oracle/reference_ops.py) against
+the reference and refuses to write fixtures if they disagree. The tests need only the committed fixtures, not the
+reference.
 
-    python oracle/gen_golden.py            # writes tests/golden/
+    FDM_B200_REFERENCE_DIR=<reference checkout> python oracle/gen_golden.py     # writes tests/golden/
 """
 import json
 import os
@@ -16,7 +16,9 @@ import types
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("FDM_B200_REFERENCE_DIR", "")
+if not os.path.isdir(REF):
+    sys.exit("usage: FDM_B200_REFERENCE_DIR=<reference checkout> python " + " ".join(sys.argv))
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = os.path.join(ROOT, "tests", "golden")
 sys.path.insert(0, ROOT)
@@ -209,7 +211,6 @@ def main():
             cols = np.arange(0, verts.shape[-1], 16)
             g[f"verts_cols_{cb_kind}"] = verts[0][:, cols].numpy()
             if verts.shape[-1] == 15069:
-                g[f"verts_lip_{cb_kind}"] = verts[0].reshape(T, -1, 3)[:, lip].reshape(T, -1).numpy()
                 g[f"lve_{cb_kind}"] = np.float64(lip_vertex_error(np.zeros_like(verts[0].numpy()), verts[0].numpy(), lip))
         np.savez_compressed(os.path.join(OUT, f"{preset}.npz"), **g)
         del fdm, ae, diff

@@ -2,16 +2,16 @@
 
 `bench.py --impl reference` and bench.py's `cpu_baseline` leg time the reference's own PyTorch implementation of the
 sampling path. The reference has no packaging (no setup.py / pyproject.toml), so it cannot be pip-installed into
-`baseline/_ref`; instead `__graft_entry__.build()` copies the reference's hot-path packages (models/, utiles/,
-video_diffusion_pytorch/: the files SURVEY.md section 8(a) cites) UNMODIFIED into `oracle/_ref/`, which is git-ignored
-but travels to the GPU box with the snapshot. This module imports them from there with the harness shims of SURVEY.md
+`baseline/_ref`; instead `__graft_entry__.build()`, given a checkout of it in FDM_B200_REFERENCE_DIR, copies the
+reference's hot-path packages (models/, utiles/, video_diffusion_pytorch/: the files SURVEY.md section 8(a) cites)
+UNMODIFIED into the git-ignored `oracle/_ref/`. This module imports them from there with the harness shims of SURVEY.md
 section 8(c) (missing optional modules stubbed, audio encoders built from their configs with random weights,
 zero-initialised output layer re-initialised) and drives them exactly as samples/sample_diffusion_*.py do: B = 1, the
 audio encoder re-run inside every denoiser call, `diffusion.p_sample` per step. Classifier-free guidance follows
 utiles/classifierfree.py:15-21 (two denoiser calls per step, the second with the null condition).
 
-When `oracle/_ref` is absent (a checkout that never ran build() next to /root/reference) callers fall back to the
-oracle port (oracle/reference_ops.py) and say so (`cpu_baseline.kind == "port"`)."""
+When `oracle/_ref` is absent (build() ran without FDM_B200_REFERENCE_DIR) callers fall back to the oracle port
+(oracle/reference_ops.py) and say so (`cpu_baseline.kind == "port"`)."""
 import os
 import sys
 import time
@@ -26,8 +26,8 @@ def available() -> bool:
     return all(os.path.isdir(os.path.join(REF_DIR, p)) for p in REF_PACKAGES)
 
 
-def install_from(src: str = "/root/reference") -> bool:
-    """Copy the reference's hot-path packages (python files only, unmodified) into oracle/_ref. Build-container only."""
+def install_from(src: str) -> bool:
+    """Copy the reference's hot-path packages (python files only, unmodified) from the checkout `src` into oracle/_ref."""
     import shutil
     if not os.path.isdir(src):
         return False
@@ -43,7 +43,7 @@ def _import_reference():
     """Import the reference modules from oracle/_ref in a way that cannot collide with the drop-in packages of the same
     names: the caller must be a process that has NOT imported face-diffusion-model_b200's `models` (bench.py runs the
     reference in a subprocess)."""
-    assert available(), "oracle/_ref is missing: run __graft_entry__.build() in the build container"
+    assert available(), "oracle/_ref is missing: run __graft_entry__.build() with FDM_B200_REFERENCE_DIR set"
     for name in ("models", "utiles", "video_diffusion_pytorch"):
         assert name not in sys.modules, f"{name} already imported: run the reference in its own process"
     sys.path.insert(0, REF_DIR)
