@@ -150,38 +150,50 @@ class DenoiserEngine:
 
     # ---- per-clip-batch state ---------------------------------------------------------------------
     def prepare(self, audio_hidden: torch.Tensor, n_frames: int, id_one_hot: torch.Tensor,
-                emo_one_hot: Optional[torch.Tensor] = None, guidance: Optional[str] = None) -> None:
-        """audio_hidden: (B, N, audio_dim) audio-encoder output in the compute dtype; n_frames: latent frames T.
+                emo_one_hot: Optional[torch.Tensor] = None, guidance: Optional[str] = None, fanout: int = 1) -> None:
+        """audio_hidden: (A, N, audio_dim) audio-encoder output in the compute dtype; n_frames: latent frames T.
+        fanout: K sequences per audio clip, B = A*K sequences, sequence a*K + k on clip a; the one-hots have B rows or 1.
         guidance: None, or the name of the condition the unconditional pass zeroes ("id" | "emotion")."""
         self.pack()
         P, w, d = self.P, self.w, self.P.d
-        B, N, Ca = audio_hidden.shape
-        assert Ca == P.audio_dim and audio_hidden.dtype == self.dtype and audio_hidden.is_contiguous()
+        A, N, Ca = audio_hidden.shape
+        assert Ca == P.audio_dim and audio_hidden.dtype == self.dtype and audio_hidden.is_contiguous() and fanout >= 1
+        B = A * fanout
         Ta = N // 2 if P.pair_audio else N
         if n_frames > Ta:
             raise ValueError(f"latent has {n_frames} frames but the audio only yields {Ta} (the reference fails here too)")
+        for oh in (id_one_hot, emo_one_hot):  # checked before any buffer changes, so a refused call keeps the prepared state
+            rows = 1 if oh is None or oh.dim() == 1 else oh.shape[0]
+            if rows not in (1, B):
+                raise ValueError(f"a condition has {rows} rows; the call has {B} sequences (give {B} rows or 1)")
         T = n_frames
         if P.pair_audio:
-            a = audio_hidden[:, : 2 * T].reshape(B, T, 2 * Ca)
+            a = audio_hidden[:, : 2 * T].reshape(A, T, 2 * Ca)
         else:
             a = audio_hidden[:, :T]
-        a = a.reshape(B * T, P.audio_in) if a.is_contiguous() else a.contiguous().view(B * T, P.audio_in)
+        a = a.reshape(A * T, P.audio_in) if a.is_contiguous() else a.contiguous().view(A * T, P.audio_in)
         dev, dt = self.dev, self.dtype
-        BT = B * T
-        h = self.buf("prep_h", (BT, d), dt)
-        af = self.buf("prep_af", (BT, d), dt)
+        AT, BT = A * T, B * T
+        h = self.buf("prep_h", (AT, d), dt)
+        af = self.buf("prep_af", (AT, d), dt)
         lib.gemm(a, w["ae0_w"], h, bias=w["ae0_b"], act=lib.ACT_MISH)
         lib.gemm(h, w["ae2_w"], af, bias=w["ae2_b"])
         af_op = lib.split(af) if self.precision == "x3" else af  # (operand of eight GEMMs: split once)
-        # audio part of the collapsed cross-attention, per layer
+        # audio part of the collapsed cross-attention, per layer and clip; with fan-out each clip's block is then copied
+        # to its K sequences, so the step reads the same (B*T, d) caches as for the repeated audio batch
+        cc = self.buf("prep_cross", (AT, d), dt) if fanout > 1 else None
         self.cross = []
         for l in range(P.layers):
             L = w[l]
             c = self.buf(f"cross{l}", (BT, d), dt)
             lib.gemm(af_op, L["cv_w"], h, bias=L["cv_b"])
-            lib.gemm(h, L["co_w"], c, bias=L["co_b"])
+            if cc is None:
+                lib.gemm(h, L["co_w"], c, bias=L["co_b"])
+            else:
+                lib.gemm(h, L["co_w"], cc, bias=L["co_b"])
+                c.view(A, fanout, T, d).copy_(cc.view(A, 1, T, d).expand(A, fanout, T, d))  # setup-time broadcast
             self.cross.append(c)
-        # style (+ emotion) per clip and pass, plus positional encoding -> one addend tensor per pass
+        # style (+ emotion) per sequence and pass, plus positional encoding -> one addend tensor per pass
         def expand(oh, n):
             oh = oh.to(dev, torch.float32)
             if oh.dim() == 1:

@@ -93,6 +93,14 @@ class _PE(nn.Module):
         self.register_buffer("pe", table)
 
 
+def fanout(n_audio: int, n_seq: int) -> int:
+    """Sequences per audio clip K of a call with `n_audio` audio rows and `n_seq` latent rows: sequence a*K + k uses
+    clip a (the order of audio.repeat_interleave(K, 0)). n_audio == n_seq is the one-sequence-per-clip call."""
+    if n_audio < 1 or n_seq % n_audio != 0:
+        raise ValueError(f"{n_seq} sequences do not split evenly over {n_audio} audio clips")
+    return n_seq // n_audio
+
+
 class FDMBase(nn.Module):
     preset_name: str = ""
 
@@ -209,7 +217,9 @@ class FDMBase(nn.Module):
         return e.pack_serial
 
     def set_audio_features(self, audio: torch.Tensor, hidden: torch.Tensor) -> None:
-        """Register precomputed audio-encoder features (B, N, audio_dim) for `audio` (skips the encoder run)."""
+        """Register precomputed audio-encoder features (A, N, audio_dim) for the (A, L) `audio` (skips the encoder run)."""
+        if hidden.shape[0] != audio.shape[0]:
+            raise ValueError(f"features for {hidden.shape[0]} clips do not match {audio.shape[0]} audio clips")
         mode = self._audio_mode()
         if hasattr(self.audio_encoder, "precision"):
             self.audio_encoder.precision = mode
@@ -221,19 +231,20 @@ class FDMBase(nn.Module):
         self.__dict__["_tail_key"] = None
 
     def prepare(self, audio, n_frames: int, id_one_hot, emo_one_hot=None, guidance: Optional[str] = None,
-                tail: bool = False) -> DenoiserEngine:
-        """Per-clip-batch state of the step engine (tail=False) or of the high-precision tail engine (tail=True)."""
+                tail: bool = False, fanout: int = 1) -> DenoiserEngine:
+        """Per-clip-batch state of the step engine (tail=False) or of the high-precision tail engine (tail=True) for
+        A = audio.shape[0] clips with `fanout` (K) sequences each; the condition one-hots have A*K rows or 1."""
         eng = self.tail_engine() if tail else self.engine()
         slot = "_tail_key" if tail else "_prep_key"
         eng.pack()
         k = self.__dict__[slot]
         hidden = self.encode_audio(audio)  # (cache hit unless the audio tensor or the encoder's weights changed)
-        meta = (n_frames, guidance, eng.pack_serial, self.__dict__.get("_audio_serial", 0))
+        meta = (n_frames, guidance, fanout, eng.pack_serial, self.__dict__.get("_audio_serial", 0))
         if k is None or k[1] != meta or not self._same(k[0], (audio, id_one_hot, emo_one_hot)) or eng.B == 0:
             if hidden.dtype != eng.dtype:  # split-bf16 audio features feeding the bf16 step engine
                 hidden = lib.cast(hidden, torch.empty_like(hidden, dtype=eng.dtype))
             with lib.nvtx_range("prepare_tail" if tail else "prepare"):
-                eng.prepare(hidden, n_frames, id_one_hot, emo_one_hot, guidance)
+                eng.prepare(hidden, n_frames, id_one_hot, emo_one_hot, guidance, fanout=fanout)
             self.__dict__[slot] = (self._ident((audio, id_one_hot, emo_one_hot)), meta)
         return eng
 
@@ -254,7 +265,7 @@ class FDMBase(nn.Module):
         B = vertice.shape[0]
         assert vertice.shape[1] % P.fq == 0 and vertice.shape[2] * P.fq == P.d, "latent must be (B, fq*T, d/fq)"
         n_frames = vertice.shape[1] // P.fq
-        eng = self.prepare(audio, n_frames, id_one_hot, emo_one_hot, guidance)
+        eng = self.prepare(audio, n_frames, id_one_hot, emo_one_hot, guidance, fanout=fanout(audio.shape[0], B))
         t_dev = torch.as_tensor(t, device=vertice.device).reshape(-1)[:1].to(torch.int32)
         x = vertice.float().contiguous().view(B * n_frames, P.d)
         if eng.dtype == torch.bfloat16:
@@ -327,6 +338,8 @@ def cosine_tables(timesteps: int, s: float = 0.008):
 
 
 class GaussianDiffusionBase(nn.Module):
+    """Sampling calls take `audio` (A, L) and a latent of B = A*K sequences: sequence a*K + k uses clip a (the order of
+    audio.repeat_interleave(K, 0)), and each clip's audio work runs once. Condition one-hots have B rows or 1."""
     n_cond: int = 1                 # 1: (id_one_hot) ; 2: (emo_one_hot, id_one_hot)
     default_range = (1000, 0)       # p_sample_loop runs t = hi-1 .. lo
 
@@ -394,12 +407,12 @@ class GaussianDiffusionBase(nn.Module):
         lib.philox_normal(x, seed, self.clip_index0, self.num_timesteps)  # step index T = "x_T draw"
         return x
 
-    def _tail(self, fdm, audio, n_frames, idh, emo, gcond, n_steps):
+    def _tail(self, fdm, audio, n_frames, idh, emo, gcond, n_steps, k):
         """(tail engine, number of high-precision tail steps) for a bf16-mode sampling call."""
         n = min(int(fdm.hi_tail_steps), n_steps) if fdm.precision == "bf16" else 0
         if n <= 0:
             return None
-        return fdm.prepare(audio, n_frames, idh, emo, guidance=gcond, tail=True), n
+        return fdm.prepare(audio, n_frames, idh, emo, guidance=gcond, tail=True, fanout=k), n
 
     # -- reference API ----------------------------------------------------------------------------------
     @torch.inference_mode()
@@ -429,9 +442,10 @@ class GaussianDiffusionBase(nn.Module):
         steps = list(range(hi - 1, lo - 1, -1)) if steps is None else [int(t) for t in steps]
         seed = self._call_seed()
         x_T = self._initial_latent(tuple(shape), device, seed) if x_T is None else x_T.to(device, torch.float32)
-        eng = fdm.prepare(audio, shape[1] // P.fq, idh, emo, guidance=gcond)
+        k = fanout(audio.shape[0], shape[0])
+        eng = fdm.prepare(audio, shape[1] // P.fq, idh, emo, guidance=gcond, fanout=k)
         sampler = SamplerEngine(eng, self.posterior_mean_coef1, self.posterior_mean_coef2, self._sigma_table(), level)
-        tail = self._tail(fdm, audio, shape[1] // P.fq, idh, emo, gcond, len(steps))
+        tail = self._tail(fdm, audio, shape[1] // P.fq, idh, emo, gcond, len(steps), k)
         with lib.nvtx_range("sampling_loop"):
             out = sampler.run(x_T, steps, noise=self.noise_source, seed=seed, clip_index0=self.clip_index0,
                               graph=self.use_cuda_graph, tap=tap, time_steps=getattr(self, "time_steps", False), tail=tail)
@@ -465,9 +479,10 @@ class GaussianDiffusionBase(nn.Module):
         tables = {k: v.to(device=device, dtype=torch.float32).contiguous() for k, v in tables.items()}
         shape = tuple(latent_motion_shape)
         x_T = self._initial_latent(shape, device, self._call_seed()) if x_T is None else x_T.to(device, torch.float32)
-        eng = fdm.prepare(audio, shape[1] // P.fq, idh, emo, guidance=gcond)
+        k = fanout(audio.shape[0], shape[0])
+        eng = fdm.prepare(audio, shape[1] // P.fq, idh, emo, guidance=gcond, fanout=k)
         sampler = SamplerEngine(eng, self.posterior_mean_coef1, self.posterior_mean_coef2, self._sigma_table(), level)
-        tail = self._tail(fdm, audio, shape[1] // P.fq, idh, emo, gcond, len(pairs))
+        tail = self._tail(fdm, audio, shape[1] // P.fq, idh, emo, gcond, len(pairs), k)
         with lib.nvtx_range("ddim_loop"):
             out = sampler.run(x_T, [p[0] for p in pairs], graph=self.use_cuda_graph, tap=tap, ddim=tables,
                               time_steps=getattr(self, "time_steps", False), tail=tail)

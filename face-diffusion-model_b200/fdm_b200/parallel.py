@@ -3,7 +3,7 @@
 One process per GPU (torchrun), weights replicated, clip b of the global batch lives on rank b // B_local; the
 in-kernel sampler noise is keyed by the GLOBAL clip index, so results do not depend on the world size. The only
 collective is one all-gather of the decoded vertex sequences (SURVEY.md §8(e)); the reference has no distributed
-code at all."""
+code at all. A fan-out call (several sequences per audio clip) shards by audio clip: fanout_shard_range."""
 from __future__ import annotations
 
 from typing import Callable, Optional, Tuple
@@ -20,6 +20,15 @@ def shard_range(n_clips: int, rank: int, world: int) -> Tuple[int, int]:
         raise ValueError(f"{n_clips} clips do not split evenly over {world} ranks (pad the batch)")
     per = n_clips // world
     return rank * per, per
+
+
+def fanout_shard_range(n_audio: int, fanout: int, rank: int, world: int) -> Tuple[Tuple[int, int], Tuple[int, int]]:
+    """Shard of a fan-out call (n_audio clips x `fanout` sequences each, sequence a*fanout + k on clip a) by audio clip, so
+    that a clip's sequences stay on one rank and its audio is encoded once: returns ((first clip, clip count), (first
+    sequence, sequence count)). The first sequence is the rank's `diffusion.clip_index0` (noise keyed by the global sequence
+    index), and the gathered (world * count, ...) sequences are in global order."""
+    a0, na = shard_range(n_audio, rank, world)
+    return (a0, na), (a0 * fanout, na * fanout)
 
 
 def gather_clips(local: torch.Tensor, group=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
