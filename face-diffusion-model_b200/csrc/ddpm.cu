@@ -151,6 +151,49 @@ __global__ void __launch_bounds__(256) ddim_step_kernel(const fdm_ddim_args a, c
   }
 }
 
+// grid = rows (one CTA per (sequence, frame) row). The mask is written by host copies before the sampling loop, never by
+// the kernels this one follows, so a CTA may read it before pdl_wait(), and a CTA of an unknown row exits without waiting,
+// except CTA 0: the grid must not complete before its predecessor has, or the next kernel's pdl_wait() (advance_cursor
+// rewriting t_dev / cursor) would no longer order it after the step update, e.g. when no row is known.
+__global__ void __launch_bounds__(128) known_frames_kernel(const fdm_known_args a, const int64_t d4) {
+  pdl_trigger();
+  const int64_t row = blockIdx.x;
+  const bool known = a.mask[row] != 0;
+  if (!known && row != 0) return;
+  pdl_wait();
+  if (!known) return;
+  const int i = *a.index_dev + a.offset;
+  const float ka = a.ka[i], kb = a.kb[i];
+  const bool draw = kb != 0.f;
+  const bool philox = draw && a.noise == nullptr;
+  const int64_t b = row / a.T;
+  const uint32_t clip = static_cast<uint32_t>(a.clip_index0 + b);
+  const uint64_t seed = philox ? *a.seed_dev : 0;
+  const uint32_t t = philox ? static_cast<uint32_t>(*a.t_dev) : 0u;
+  const int64_t e4_0 = (row - b * a.T) * d4;  // first float4 of the row within its sequence (the Philox element counter)
+  for (int64_t j = threadIdx.x; j < d4; j += blockDim.x) {
+    const int64_t i4 = row * d4 + j;
+    const float4 k = reinterpret_cast<const float4*>(a.known)[i4];
+    float4 o = make_float4(__fmul_rn(ka, k.x), __fmul_rn(ka, k.y), __fmul_rn(ka, k.z), __fmul_rn(ka, k.w));
+    if (draw) {
+      const float4 z = philox ? philox_normal4(seed, clip, t, static_cast<uint64_t>(e4_0 + j))
+                              : reinterpret_cast<const float4*>(a.noise)[i4];
+      o.x = __fadd_rn(o.x, __fmul_rn(kb, z.x));
+      o.y = __fadd_rn(o.y, __fmul_rn(kb, z.y));
+      o.z = __fadd_rn(o.z, __fmul_rn(kb, z.z));
+      o.w = __fadd_rn(o.w, __fmul_rn(kb, z.w));
+    }
+    reinterpret_cast<float4*>(a.x)[i4] = o;
+    if (a.x_bf16) {
+      uint2 u;
+      __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&u);
+      h[0] = __floats2bfloat162_rn(o.x, o.y);
+      h[1] = __floats2bfloat162_rn(o.z, o.w);
+      reinterpret_cast<uint2*>(a.x_bf16)[i4] = u;
+    }
+  }
+}
+
 __global__ void advance_cursor_kernel(int32_t* cursor, const int32_t* sched, int n, int32_t* t_dev) {
   pdl_trigger();
   pdl_wait();
@@ -209,6 +252,20 @@ extern "C" int fdm_ddim_step(const fdm_ddim_args* args, void* stream) {
   FDM_CHECK_ARG(al % 16 == 0 && reinterpret_cast<uintptr_t>(a.out_bf16) % 8 == 0, "fdm_ddim_step: operands must be 16-byte aligned");
   FDM_CHECK_CUDA(fdm_launch_pdl(ddim_step_kernel, dim3(grid_for(a.n / 4)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), 1, a,
                                 a.n / 4));
+  return 0;
+}
+
+extern "C" int fdm_known_frames(const fdm_known_args* args, void* stream) {
+  FDM_CHECK_ARG(args != nullptr, "fdm_known_frames: null args");
+  const fdm_known_args& a = *args;
+  FDM_CHECK_ARG(a.x && a.known && a.mask && a.ka && a.kb && a.index_dev, "fdm_known_frames: null operand");
+  FDM_CHECK_ARG(a.noise || (a.seed_dev && a.t_dev), "fdm_known_frames: need noise or seed_dev and t_dev");
+  FDM_CHECK_ARG(a.B > 0 && a.T > 0 && a.d > 0 && a.d % 4 == 0, "fdm_known_frames: need B, T > 0 and d a positive multiple of 4");
+  FDM_CHECK_ARG(a.B * a.T <= 0x7fffffff, "fdm_known_frames: at most 2^31 - 1 rows per call");
+  const uintptr_t al = reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.known) | reinterpret_cast<uintptr_t>(a.noise);
+  FDM_CHECK_ARG(al % 16 == 0 && reinterpret_cast<uintptr_t>(a.x_bf16) % 8 == 0, "fdm_known_frames: operands must be 16-byte aligned");
+  FDM_CHECK_CUDA(fdm_launch_pdl(known_frames_kernel, dim3(static_cast<unsigned>(a.B * a.T)), dim3(128), 0,
+                                reinterpret_cast<cudaStream_t>(stream), 1, a, a.d / 4));
   return 0;
 }
 

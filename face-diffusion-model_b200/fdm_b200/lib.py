@@ -56,6 +56,12 @@ class DdimArgs(C.Structure):
                 ("a_recip", _vp), ("a_recipm1", _vp), ("sqrt_an", _vp), ("c", _vp), ("index_dev", _vp), ("n", _i64)]
 
 
+class KnownArgs(C.Structure):
+    _fields_ = [("x", _vp), ("x_bf16", _vp), ("known", _vp), ("mask", _vp), ("noise", _vp), ("ka", _vp), ("kb", _vp),
+                ("index_dev", _vp), ("offset", _i32), ("seed_dev", _vp), ("t_dev", _vp), ("clip_index0", _i64),
+                ("B", _i64), ("T", _i64), ("d", _i64)]
+
+
 EXPORTS = {
     "fdm_last_error": (C.c_char_p, []),
     "fdm_device_info": (C.c_int, [C.POINTER(_i32)] * 3),
@@ -69,6 +75,7 @@ EXPORTS = {
     "fdm_self_attention": (C.c_int, [C.POINTER(AttnArgs), _vp]),
     "fdm_ddpm_step": (C.c_int, [C.POINTER(DdpmArgs), _vp]),
     "fdm_ddim_step": (C.c_int, [C.POINTER(DdimArgs), _vp]),
+    "fdm_known_frames": (C.c_int, [C.POINTER(KnownArgs), _vp]),
     "fdm_advance_cursor": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "fdm_philox_normal": (C.c_int, [_vp, _i64, _i64, _u64, _i64, _i32, _vp]),
     "fdm_vq_quantize": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),
@@ -105,7 +112,11 @@ def load() -> C.CDLL:
                            "(there is no CPU fallback)")
         lib = C.CDLL(LIB_PATH)
         for name, (res, args) in EXPORTS.items():
-            fn = getattr(lib, name)
+            try:
+                fn = getattr(lib, name)
+            except AttributeError:  # a library built from older sources
+                raise FdmError(f"{LIB_PATH} does not export {name}: rebuild it "
+                               "(`python -c 'import __graft_entry__ as g; g.build()'`)") from None
             fn.restype, fn.argtypes = res, args
         if lib.fdm_abi_version() != ABI_VERSION:  # a stale build would read the argument structs with another layout
             raise FdmError(f"{LIB_PATH} has ABI version {lib.fdm_abi_version()}, this binding needs {ABI_VERSION}: rebuild it "
@@ -419,6 +430,33 @@ def ddim_step(x0_cond, x_t, out, a_recip, a_recipm1, sqrt_an, c, index_dev, *, x
     _check(lib.fdm_ddim_step(C.byref(a), _stream()))
     _launched()
     return out
+
+
+def known_frames(x, known, mask, ka, kb, index_dev, *, offset: int = 0, noise=None, x_bf16=None,
+                 seed_dev: Optional[torch.Tensor] = None, t_dev: Optional[torch.Tensor] = None, clip_index0: int = 0) -> torch.Tensor:
+    """Known-frame replacement in place (fdm_known_frames): x (B, ...) fp32 holds B sequences of mask.numel() / B rows;
+    rows whose uint8 mask is set become ka[i] * known + kb[i] * z with i = index_dev[0] + offset, z from `noise` (may be
+    x itself) or, when noise is None, the Philox draw of (seed_dev[0], clip_index0 + b, t_dev[0], element)."""
+    lib = require_device()
+    a = KnownArgs()
+    B, rows = x.shape[0], mask.numel()
+    for t in (x, known, noise):
+        assert t is None or (t.dtype == torch.float32 and t.is_contiguous() and t.numel() == x.numel())
+    assert mask.dtype == torch.uint8 and mask.is_contiguous() and rows % B == 0 and x.numel() % rows == 0
+    assert ka.dtype == kb.dtype == torch.float32 and index_dev.dtype == torch.int32
+    if x_bf16 is not None:
+        assert x_bf16.dtype == torch.bfloat16 and x_bf16.is_contiguous() and x_bf16.numel() == x.numel()
+    if seed_dev is not None:
+        assert seed_dev.dtype == torch.int64 and seed_dev.numel() == 1
+    if t_dev is not None:
+        assert t_dev.dtype == torch.int32 and t_dev.numel() == 1
+    a.x, a.x_bf16, a.known, a.mask, a.noise = _ptr(x), _ptr(x_bf16), _ptr(known), _ptr(mask), _ptr(noise)
+    a.ka, a.kb, a.index_dev, a.offset = _ptr(ka), _ptr(kb), _ptr(index_dev), offset
+    a.seed_dev, a.t_dev, a.clip_index0 = _ptr(seed_dev), _ptr(t_dev), clip_index0
+    a.B, a.T, a.d = B, rows // B, x.numel() // rows
+    _check(lib.fdm_known_frames(C.byref(a), _stream()))
+    _launched()
+    return x
 
 
 def advance_cursor(cursor: torch.Tensor, t_sched: torch.Tensor, t_dev: torch.Tensor) -> None:

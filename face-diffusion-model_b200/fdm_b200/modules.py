@@ -19,7 +19,7 @@ from . import lib
 from .audio import AudioEncoderEngine
 from .denoiser import DenoiserEngine, _sin_table
 from .presets import PRESETS, Preset
-from .sampler import SamplerEngine
+from .sampler import SamplerEngine, pool_known
 from .vqvae import VQDecoderEngine, quantize
 
 DEFAULT_PRECISION = os.environ.get("FDM_B200_PRECISION", "bf16")
@@ -339,7 +339,13 @@ def cosine_tables(timesteps: int, s: float = 0.008):
 
 class GaussianDiffusionBase(nn.Module):
     """Sampling calls take `audio` (A, L) and a latent of B = A*K sequences: sequence a*K + k uses clip a (the order of
-    audio.repeat_interleave(K, 0)), and each clip's audio work runs once. Condition one-hots have B rows or 1."""
+    audio.repeat_interleave(K, 0)), and each clip's audio work runs once. Condition one-hots have B rows or 1.
+
+    Known frames (p_sample_loop / sample / ddim_sample): `known` (B or 1, fq*T, zdim) float32, the layout
+    VQAutoEncoder.encode returns, and `known_mask` bool (B, T) or (T,), one entry per frame. Masked frames start from
+    sqrt_alphas_cumprod[t0] * known + sqrt_one_minus_alphas_cumprod[t0] * x_T and are put back on the forward process
+    after every step (the draw of that step's update as noise); after the last step they hold `known` bit for bit, and
+    the other frames are sampled around them."""
     n_cond: int = 1                 # 1: (id_one_hot) ; 2: (emo_one_hot, id_one_hot)
     default_range = (1000, 0)       # p_sample_loop runs t = hi-1 .. lo
 
@@ -414,6 +420,42 @@ class GaussianDiffusionBase(nn.Module):
             return None
         return fdm.prepare(audio, n_frames, idh, emo, guidance=gcond, tail=True, fanout=k), n
 
+    @staticmethod
+    def _check_known(shape, P, known, known_mask):
+        """None, or (known, mask) broadcastable to the call's (B, fq*T, zdim) latent and (B, T) frames. Raises ValueError
+        before any device state changes."""
+        if known is None and known_mask is None:
+            return None
+        if known is None or known_mask is None:
+            raise ValueError("known and known_mask go together: give both or neither")
+        B, L, z = shape
+        T = L // P.fq
+        if not isinstance(known, torch.Tensor) or known.dtype != torch.float32:
+            raise ValueError(f"known must be a float32 tensor (the latent autoencoder.encode returns), got "
+                             f"{getattr(known, 'dtype', type(known).__name__)}")
+        if known.dim() != 3 or known.shape[0] not in (1, B) or tuple(known.shape[1:]) != (L, z):
+            raise ValueError(f"known has shape {tuple(known.shape)}; the call needs ({B} or 1, {L}, {z})")
+        if not isinstance(known_mask, torch.Tensor) or known_mask.dtype != torch.bool:
+            raise ValueError(f"known_mask must be a bool tensor, got {getattr(known_mask, 'dtype', type(known_mask).__name__)}")
+        if tuple(known_mask.shape) not in ((B, T), (T,)):
+            raise ValueError(f"known_mask has shape {tuple(known_mask.shape)}; the call has {B} sequences of {T} frames "
+                             f"(give ({B}, {T}) or ({T},))")
+        return known, known_mask
+
+    def _known_tables(self, steps: Sequence[int], ddim: Optional[dict] = None):
+        """(ka, kb) fp32 host tables of a call with known frames, len(steps) + 1 entries: entry 0 the start at the noise level
+        of the first step, entry s + 1 the state after step s (DDPM: noise level t - 1; DDIM: the step's host tables
+        sqrt_an / c), the last entry (1, 0)."""
+        sa, sb = self.sqrt_alphas_cumprod.detach().cpu(), self.sqrt_one_minus_alphas_cumprod.detach().cpu()
+        if ddim is None:
+            prev = torch.tensor([t - 1 for t in steps[:-1]], dtype=torch.long)
+            ka_mid = torch.where(prev >= 0, sa[prev.clamp(min=0)], torch.ones(()))
+            kb_mid = torch.where(prev >= 0, sb[prev.clamp(min=0)], torch.zeros(()))
+        else:
+            ka_mid, kb_mid = ddim["sqrt_an"][:-1].float(), ddim["c"][:-1].float()
+        t0 = int(steps[0])
+        return (torch.cat([sa[t0:t0 + 1], ka_mid, torch.ones(1)]), torch.cat([sb[t0:t0 + 1], kb_mid, torch.zeros(1)]))
+
     # -- reference API ----------------------------------------------------------------------------------
     @torch.inference_mode()
     def p_sample(self, x, t, audio, *conds, clip_denoised=False, noise=None):
@@ -433,27 +475,32 @@ class GaussianDiffusionBase(nn.Module):
 
     @torch.inference_mode()
     def p_sample_loop(self, shape, audio, *conds, x_T: Optional[torch.Tensor] = None,
-                      step_range: Optional[Sequence[int]] = None, steps: Optional[Sequence[int]] = None, tap=None):
+                      step_range: Optional[Sequence[int]] = None, steps: Optional[Sequence[int]] = None, tap=None,
+                      known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None):
         device = self.betas.device
         idh, emo = self._split(conds)
         fdm, level, gcond = self._fdm()
         P = fdm.preset
         hi, lo = step_range if step_range is not None else self.default_range
         steps = list(range(hi - 1, lo - 1, -1)) if steps is None else [int(t) for t in steps]
+        kn = self._check_known(tuple(shape), P, known, known_mask)
         seed = self._call_seed()
         x_T = self._initial_latent(tuple(shape), device, seed) if x_T is None else x_T.to(device, torch.float32)
         k = fanout(audio.shape[0], shape[0])
         eng = fdm.prepare(audio, shape[1] // P.fq, idh, emo, guidance=gcond, fanout=k)
         sampler = SamplerEngine(eng, self.posterior_mean_coef1, self.posterior_mean_coef2, self._sigma_table(), level)
         tail = self._tail(fdm, audio, shape[1] // P.fq, idh, emo, gcond, len(steps), k)
+        kf = None if kn is None else pool_known(eng, *kn, *self._known_tables(steps))
         with lib.nvtx_range("sampling_loop"):
             out = sampler.run(x_T, steps, noise=self.noise_source, seed=seed, clip_index0=self.clip_index0,
-                              graph=self.use_cuda_graph, tap=tap, time_steps=getattr(self, "time_steps", False), tail=tail)
+                              graph=self.use_cuda_graph, tap=tap, time_steps=getattr(self, "time_steps", False), tail=tail,
+                              known=kf)
         self.__dict__["_last_sampler"] = sampler
         return out
 
     @torch.inference_mode()
-    def ddim_sample(self, audio, latent_motion_shape, *conds_and_steps, x_T: Optional[torch.Tensor] = None, tap=None):
+    def ddim_sample(self, audio, latent_motion_shape, *conds_and_steps, x_T: Optional[torch.Tensor] = None, tap=None,
+                    known: Optional[torch.Tensor] = None, known_mask: Optional[torch.Tensor] = None):
         """Deterministic DDIM sampling, eta = 0 (reference diffusion_BIWI_encoder_decoder.py:675-710):
         ddim_sample(audio, shape, id_one_hot, steps=500). The reference's last time pair (t, -1) evaluates the
         denoiser and then leaves the sample unchanged; that evaluation is skipped here."""
@@ -465,6 +512,8 @@ class GaussianDiffusionBase(nn.Module):
         idh, emo = self._split(conds)
         fdm, level, gcond = self._fdm()
         P = fdm.preset
+        shape = tuple(latent_motion_shape)
+        kn = self._check_known(shape, P, known, known_mask)
         times = list(reversed(np.linspace(-1, 1000 - 1, n_steps + 1).astype(np.int32).tolist()))
         pairs = [(i, j) for i, j in zip(times[:-1], times[1:]) if j >= 0]
         t_cur = torch.tensor([p[0] for p in pairs], dtype=torch.long)
@@ -476,16 +525,20 @@ class GaussianDiffusionBase(nn.Module):
         tables = {"a_recip": self.sqrt_recip_alphas_cumprod.detach().cpu()[t_cur],
                   "a_recipm1": self.sqrt_recipm1_alphas_cumprod.detach().cpu()[t_cur],
                   "sqrt_an": torch.sqrt(an), "c": torch.sqrt(1 - an - sigma ** 2)}
+        known_ab = None if kn is None else self._known_tables([p[0] for p in pairs], tables)
         tables = {k: v.to(device=device, dtype=torch.float32).contiguous() for k, v in tables.items()}
-        shape = tuple(latent_motion_shape)
-        x_T = self._initial_latent(shape, device, self._call_seed()) if x_T is None else x_T.to(device, torch.float32)
+        seed = self._call_seed() if x_T is None or kn is not None else None
+        x_T = self._initial_latent(shape, device, seed) if x_T is None else x_T.to(device, torch.float32)
         k = fanout(audio.shape[0], shape[0])
         eng = fdm.prepare(audio, shape[1] // P.fq, idh, emo, guidance=gcond, fanout=k)
         sampler = SamplerEngine(eng, self.posterior_mean_coef1, self.posterior_mean_coef2, self._sigma_table(), level)
         tail = self._tail(fdm, audio, shape[1] // P.fq, idh, emo, gcond, len(pairs), k)
+        # with known frames the replacement draws Philox at (call seed, clip_index0 + b, t_cur); without, the call keeps
+        # the sampler's default seed / clip_index0 (and so its cached graphs)
+        kw = {} if kn is None else dict(seed=seed, clip_index0=self.clip_index0, known=pool_known(eng, *kn, *known_ab))
         with lib.nvtx_range("ddim_loop"):
             out = sampler.run(x_T, [p[0] for p in pairs], graph=self.use_cuda_graph, tap=tap, ddim=tables,
-                              time_steps=getattr(self, "time_steps", False), tail=tail)
+                              time_steps=getattr(self, "time_steps", False), tail=tail, **kw)
         self.__dict__["_last_sampler"] = sampler
         return out
 

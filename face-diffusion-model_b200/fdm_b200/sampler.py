@@ -9,7 +9,7 @@ touches the host, so the whole step is captured once and replayed for every t.
 from __future__ import annotations
 
 import os
-from typing import Callable, Optional, Sequence, Union
+from typing import Callable, NamedTuple, Optional, Sequence, Union
 
 import torch
 
@@ -17,6 +17,30 @@ from . import lib
 from .denoiser import DenoiserEngine
 
 NoiseSpec = Union[None, str, Callable[[int], torch.Tensor]]
+
+
+class KnownFrames(NamedTuple):
+    """Known frames of a sampling call, in pooled buffers of the denoiser engine (stable addresses: new known data of the
+    same shape is no reason to capture new step graphs). Rows whose mask is set take ka[s] * latent + kb[s] * z at state s
+    (0 = start, s + 1 = after step s; the last entry is (1, 0)), see fdm_known_frames."""
+    latent: torch.Tensor  # (B, fq*T, zdim) fp32
+    mask: torch.Tensor    # (B*T,) uint8, one entry per frame (denoiser row)
+    ka: torch.Tensor      # (len(steps) + 1,) fp32
+    kb: torch.Tensor
+
+
+def pool_known(den: DenoiserEngine, latent: torch.Tensor, mask: torch.Tensor, ka: torch.Tensor, kb: torch.Tensor) -> KnownFrames:
+    """Copy a call's known frames (latent broadcastable to (den.B, fq*T, zdim), mask to (den.B, den.T), host tables)
+    into the engine's pooled buffers."""
+    B, T, d = den.B, den.T, den.P.d
+    dev = den.dev
+    lat = den.buf("smp_known", (B, T * den.P.fq, d // den.P.fq), torch.float32, dev)
+    lat.copy_(latent)
+    m = den.buf("smp_known_mask", (B * T,), torch.uint8, dev)
+    m.view(B, T).copy_(mask)
+    kab = den.buf("smp_known_ab", (2, ka.numel()), torch.float32, dev)
+    kab.copy_(torch.stack([ka, kb]).to(torch.float32))
+    return KnownFrames(lat, m, kab[0], kab[1])
 
 
 class SamplerEngine:
@@ -43,7 +67,8 @@ class SamplerEngine:
     @torch.no_grad()
     def run(self, x_T: torch.Tensor, steps: Sequence[int], noise: NoiseSpec = "philox", seed: int = 0,
             clip_index0: int = 0, graph: bool = True, tap: Optional[Callable[[int, torch.Tensor], None]] = None,
-            time_steps: bool = False, ddim: Optional[dict] = None, tail=None) -> torch.Tensor:
+            time_steps: bool = False, ddim: Optional[dict] = None, tail=None,
+            known: Optional[KnownFrames] = None) -> torch.Tensor:
         """x_T (B, fq*T, zdim) fp32 on device; steps: the t values in execution order (e.g. 999..0).
         noise: "philox" (in-kernel counter-based generator), or a callable t -> tensor (host- or device-side,
         same shape as x_T) that is copied in before every step with t > 0 (parity runs).
@@ -51,7 +76,11 @@ class SamplerEngine:
         entry per element of `steps`) for the deterministic DDIM update (eta = 0, no noise).
         tail: None, or (DenoiserEngine prepared for the same clip batch, n): the LAST n steps evaluate the denoiser on that
         (high-precision, fp32-activation) engine, eagerly, after the graph-replayed bf16 steps - the final latent is the
-        last denoiser output, so its precision is what the quantiser sees (profiles/r02_precision_probe.json)."""
+        last denoiser output, so its precision is what the quantiser sees (profiles/r02_precision_probe.json).
+        known: None, or KnownFrames (pool_known): the start state and the state after every step are replaced on the known
+        rows (one fdm_known_frames launch after each step's update). Its z is the draw the update used at that element:
+        the host noise buffer, or Philox at (seed, clip_index0 + b, t); after the last step the known rows hold
+        `known.latent` bit for bit."""
         den = self.den
         B, T, d, S = den.B, den.T, den.P.d, den.passes
         assert x_T.is_cuda and x_T.dtype == torch.float32 and x_T.numel() == B * T * d, "x_T does not match prepare()"
@@ -75,6 +104,12 @@ class SamplerEngine:
         host_noise = callable(noise) and ddim is None
         noise_buf = den.buf("smp_noise", tuple(x_T.shape), torch.float32, dev) if host_noise else None
         assert host_noise or ddim is not None or noise in (None, "philox")
+        if known is not None:
+            assert known.latent.shape == x.shape and known.mask.numel() == B * T and known.ka.numel() == len(steps) + 1
+
+        def replace_known(offset: int, z=None):
+            lib.known_frames(x, known.latent, known.mask, known.ka, known.kb, cursor, offset=offset, noise=z, x_bf16=xin_bf,
+                             seed_dev=seed_dev, t_dev=t_dev, clip_index0=clip_index0)
 
         def step_body(hi: bool = False):
             x0 = tail_den.denoise(x.view(B * T, d), t_dev) if hi else den.denoise(xin, t_dev)
@@ -86,6 +121,8 @@ class SamplerEngine:
                 lib.ddim_step(x0[0], x, x, ddim["a_recip"], ddim["a_recipm1"], ddim["sqrt_an"], ddim["c"], cursor,
                               x0_uncond=x0[1] if S == 2 else None, guidance=float(self.level) if S == 2 else 0.0,
                               out_bf16=xin_bf)
+            if known is not None:  # state after step `cursor`: table entry cursor + 1
+                replace_known(1, noise_buf)
             lib.advance_cursor(cursor, sched, t_dev)
 
         def reset():
@@ -94,6 +131,8 @@ class SamplerEngine:
                 lib.cast(x, xin_bf.view(x.shape))
             cursor.zero_()
             t_dev.copy_(sched[:1])
+            if known is not None:  # start state at the first step's noise level, from x_T's own values
+                replace_known(0, x)
 
         def feed_noise(t):
             if host_noise and t > 0:
@@ -122,6 +161,8 @@ class SamplerEngine:
                    self.sigma.data_ptr(), den.x.data_ptr(), den.qkv.data_ptr(), den.att.data_ptr(), den.proj.data_ptr(),
                    den.ffn.data_ptr(), den.x0.data_ptr(), tuple(c.data_ptr() for c in den.cross),
                    tuple(a.data_ptr() for a in den.addend))
+            if known is not None:
+                key += (known.latent.data_ptr(), known.mask.data_ptr(), known.ka.data_ptr(), known.kb.data_ptr())
             hit = den.graph_cache.get(key)
             if hit is None:
                 reset()

@@ -210,6 +210,25 @@ typedef struct fdm_ddim_args {
 } fdm_ddim_args;
 int fdm_ddim_step(const fdm_ddim_args* args, void* stream);
 
+/* Known frames (latent inpainting / continuation): for every row r = b*T + f (sequence b, frame f, d elements) whose
+ * mask[r] is non-zero, with i = *index_dev + offset:
+ *   x = ka[i] * known + kb[i] * z      (each product rounded, then added: the reference's q_sample expression)
+ *   x = ka[i] * known                  (when kb[i] == 0; no draw)
+ * Rows whose mask is zero are not touched. z is noise[...] (noise may alias x: the start state reuses x_T's own value),
+ * or, when noise == NULL, the Philox normal fdm_ddpm_step draws for (seed = *seed_dev, clip_index0 + b, t = *t_dev,
+ * element) - bit-identical to fdm_philox_normal at that key. x_bf16 (optional) receives the bf16 copy of the rows
+ * written. ka / kb are per-call tables (entry 0: the start state, entry s + 1: the state after step s). */
+typedef struct fdm_known_args {
+  float* x; void* x_bf16;
+  const float* known; const uint8_t* mask;
+  const float* noise;
+  const float* ka; const float* kb;
+  const int32_t* index_dev; int32_t offset;
+  const uint64_t* seed_dev; const int32_t* t_dev; int64_t clip_index0;
+  int64_t B; int64_t T; int64_t d;   /* B sequences of T rows of d elements; x / known / noise hold B*T*d floats */
+} fdm_known_args;
+int fdm_known_frames(const fdm_known_args* args, void* stream);
+
 /* End of a graph-replayed step: cursor[0] += 1; t_dev[0] = t_sched[min(cursor[0], n_sched-1)]. */
 int fdm_advance_cursor(int32_t* cursor_dev, const int32_t* t_sched, int32_t n_sched, int32_t* t_dev, void* stream);
 /* Fill out[B*elems_per_clip] with the same Philox normals the fused step would draw for step t. */
