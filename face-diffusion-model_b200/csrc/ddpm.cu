@@ -80,14 +80,18 @@ __device__ __forceinline__ void ddpm_store(const fdm_ddpm_args& a, int64_t i, fl
   }
 }
 
-__global__ void __launch_bounds__(256) ddpm_step_kernel(const fdm_ddpm_args a, const int64_t e4_per_clip) {
+// key_clip / key_e4 (fdm_noise_keys, both or neither): the Philox draw of sequence b is keyed by (key_clip[b], key_e4[b] + e)
+// instead of (clip_index0 + b, e); fdm_ddpm_step passes nulls.
+__global__ void __launch_bounds__(256) ddpm_step_kernel(const fdm_ddpm_args a, const int64_t e4_per_clip,
+                                                        const int64_t* __restrict__ key_clip, const int64_t* __restrict__ key_e4) {
   pdl_trigger();
   pdl_wait();
   const int64_t b = blockIdx.y;
   const int t = a.t_per_clip ? static_cast<int>(a.t_per_clip[b]) : *a.t_dev;
   const float c1 = a.c1[t], c2 = a.c2[t], sg = a.sigma[t];
   const bool add_noise = t > 0;
-  const uint32_t clip = static_cast<uint32_t>(a.clip_index0 + b);
+  const uint32_t clip = static_cast<uint32_t>(key_clip ? key_clip[b] : a.clip_index0 + b);
+  const int64_t e4_key = key_e4 ? key_e4[b] : 0;
   const uint64_t seed = a.seed_dev ? *a.seed_dev : a.seed;  // device-resident seed: one captured graph, a fresh seed per call
   const int64_t base = b * e4_per_clip;
   const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
@@ -108,8 +112,8 @@ __global__ void __launch_bounds__(256) ddpm_step_kernel(const fdm_ddpm_args a, c
         za = reinterpret_cast<const float4*>(a.noise)[i0];
         zb = reinterpret_cast<const float4*>(a.noise)[i1];
       } else {
-        za = philox_normal4(seed, clip, static_cast<uint32_t>(t), static_cast<uint64_t>(e0));
-        if (two) zb = philox_normal4(seed, clip, static_cast<uint32_t>(t), static_cast<uint64_t>(e1));
+        za = philox_normal4(seed, clip, static_cast<uint32_t>(t), static_cast<uint64_t>(e4_key + e0));
+        if (two) zb = philox_normal4(seed, clip, static_cast<uint32_t>(t), static_cast<uint64_t>(e4_key + e1));
       }
     }
     ddpm_store(a, i0, ddpm_update(a, xa, ua, ta, c1, c2), za, sg, add_noise);
@@ -194,6 +198,45 @@ __global__ void __launch_bounds__(128) known_frames_kernel(const fdm_known_args 
   }
 }
 
+// grid = A * (n_w - 1) * K * O: one CTA per overlap row pair, j fastest. Both rows are read before either is written, by the
+// same thread and float4, so the pair ends bit-identical.
+__global__ void __launch_bounds__(128) window_blend_kernel(const fdm_window_args a, const int64_t d4) {
+  pdl_trigger();
+  pdl_wait();
+  const int64_t O = a.W - a.S;
+  int64_t r = blockIdx.x;
+  const int64_t j = r % O;
+  r /= O;
+  const int64_t k = r % a.K;
+  r /= a.K;
+  const int64_t w = r % (a.n_w - 1);
+  const int64_t clip = r / (a.n_w - 1);
+  const int64_t seq_lo = (clip * a.n_w + w) * a.K + k;
+  const int64_t lo = (seq_lo * a.W + a.S + j) * d4;     // row S + j of window w
+  const int64_t hi = ((seq_lo + a.K) * a.W + j) * d4;   // row j of window w + 1
+  const float lam = a.lambda[j];
+  const float mu = __fsub_rn(1.f, lam);
+  for (int64_t i = threadIdx.x; i < d4; i += blockDim.x) {
+    const float4 p = reinterpret_cast<const float4*>(a.x)[lo + i];
+    const float4 q = reinterpret_cast<const float4*>(a.x)[hi + i];
+    float4 o;
+    o.x = __fadd_rn(__fmul_rn(mu, p.x), __fmul_rn(lam, q.x));
+    o.y = __fadd_rn(__fmul_rn(mu, p.y), __fmul_rn(lam, q.y));
+    o.z = __fadd_rn(__fmul_rn(mu, p.z), __fmul_rn(lam, q.z));
+    o.w = __fadd_rn(__fmul_rn(mu, p.w), __fmul_rn(lam, q.w));
+    reinterpret_cast<float4*>(a.x)[lo + i] = o;
+    reinterpret_cast<float4*>(a.x)[hi + i] = o;
+    if (a.x_bf16) {
+      uint2 u;
+      __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&u);
+      h[0] = __floats2bfloat162_rn(o.x, o.y);
+      h[1] = __floats2bfloat162_rn(o.z, o.w);
+      reinterpret_cast<uint2*>(a.x_bf16)[lo + i] = u;
+      reinterpret_cast<uint2*>(a.x_bf16)[hi + i] = u;
+    }
+  }
+}
+
 __global__ void advance_cursor_kernel(int32_t* cursor, const int32_t* sched, int n, int32_t* t_dev) {
   pdl_trigger();
   pdl_wait();
@@ -220,7 +263,7 @@ inline int grid_for(int64_t n4) {
 
 }  // namespace
 
-extern "C" int fdm_ddpm_step(const fdm_ddpm_args* args, void* stream) {
+extern "C" int fdm_ddpm_step_keyed(const fdm_ddpm_args* args, const fdm_noise_keys* keys, void* stream) {
   FDM_CHECK_ARG(args != nullptr, "fdm_ddpm_step: null args");
   const fdm_ddpm_args& a = *args;
   FDM_CHECK_ARG(a.x0_cond && a.x_t && a.out && a.c1 && a.c2 && a.sigma, "fdm_ddpm_step: null operand");
@@ -231,6 +274,9 @@ extern "C" int fdm_ddpm_step(const fdm_ddpm_args* args, void* stream) {
                        reinterpret_cast<uintptr_t>(a.out);
   FDM_CHECK_ARG(al % 16 == 0 && reinterpret_cast<uintptr_t>(a.out_bf16) % 8 == 0, "fdm_ddpm_step: operands must be 16-byte aligned");
   FDM_CHECK_ARG(a.B <= 65535, "fdm_ddpm_step: at most 65535 clips per call");
+  const int64_t* key_clip = keys ? keys->clip : nullptr;
+  const int64_t* key_e4 = keys ? keys->e4_offset : nullptr;
+  FDM_CHECK_ARG((key_clip == nullptr) == (key_e4 == nullptr), "fdm_ddpm_step_keyed: give both key arrays or neither");
   const int64_t e4 = a.elems_per_clip / 4;
   // ~8 resident 256-thread CTAs per SM over the whole batch, two float4 per thread and iteration
   int64_t gx = ceil_div64(static_cast<int64_t>(fdm_sm_count()) * 8, a.B);
@@ -238,7 +284,25 @@ extern "C" int fdm_ddpm_step(const fdm_ddpm_args* args, void* stream) {
   if (gx > gx_max) gx = gx_max;
   if (gx < 1) gx = 1;
   FDM_CHECK_CUDA(fdm_launch_pdl(ddpm_step_kernel, dim3(static_cast<unsigned>(gx), static_cast<unsigned>(a.B)), dim3(256), 0,
-                                reinterpret_cast<cudaStream_t>(stream), 1, a, e4));
+                                reinterpret_cast<cudaStream_t>(stream), 1, a, e4, key_clip, key_e4));
+  return 0;
+}
+
+extern "C" int fdm_ddpm_step(const fdm_ddpm_args* args, void* stream) { return fdm_ddpm_step_keyed(args, nullptr, stream); }
+
+extern "C" int fdm_window_blend(const fdm_window_args* args, void* stream) {
+  FDM_CHECK_ARG(args != nullptr, "fdm_window_blend: null args");
+  const fdm_window_args& a = *args;
+  FDM_CHECK_ARG(a.x && a.lambda, "fdm_window_blend: null operand");
+  FDM_CHECK_ARG(a.A > 0 && a.n_w > 0 && a.K > 0 && a.d > 0 && a.d % 4 == 0, "fdm_window_blend: need A, n_w, K > 0 and d a positive multiple of 4");
+  FDM_CHECK_ARG(a.S > 0 && a.S < a.W && 2 * (a.W - a.S) <= a.W, "fdm_window_blend: need 0 < W - S <= W / 2");
+  const uintptr_t al = reinterpret_cast<uintptr_t>(a.x);
+  FDM_CHECK_ARG(al % 16 == 0 && reinterpret_cast<uintptr_t>(a.x_bf16) % 8 == 0, "fdm_window_blend: operands must be 16-byte aligned");
+  if (a.n_w == 1) return 0;
+  const int64_t ctas = a.A * (a.n_w - 1) * a.K * (a.W - a.S);
+  FDM_CHECK_ARG(ctas <= 0x7fffffff, "fdm_window_blend: at most 2^31 - 1 overlap rows per call");
+  FDM_CHECK_CUDA(fdm_launch_pdl(window_blend_kernel, dim3(static_cast<unsigned>(ctas)), dim3(128), 0,
+                                reinterpret_cast<cudaStream_t>(stream), 1, a, a.d / 4));
   return 0;
 }
 

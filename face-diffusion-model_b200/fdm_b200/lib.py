@@ -62,6 +62,15 @@ class KnownArgs(C.Structure):
                 ("B", _i64), ("T", _i64), ("d", _i64)]
 
 
+class NoiseKeys(C.Structure):
+    _fields_ = [("clip", _vp), ("e4_offset", _vp)]
+
+
+class WindowArgs(C.Structure):
+    _fields_ = [("x", _vp), ("x_bf16", _vp), ("lambda", _vp), ("A", _i64), ("n_w", _i64), ("K", _i64), ("W", _i64),
+                ("S", _i64), ("d", _i64)]
+
+
 EXPORTS = {
     "fdm_last_error": (C.c_char_p, []),
     "fdm_device_info": (C.c_int, [C.POINTER(_i32)] * 3),
@@ -76,6 +85,8 @@ EXPORTS = {
     "fdm_ddpm_step": (C.c_int, [C.POINTER(DdpmArgs), _vp]),
     "fdm_ddim_step": (C.c_int, [C.POINTER(DdimArgs), _vp]),
     "fdm_known_frames": (C.c_int, [C.POINTER(KnownArgs), _vp]),
+    "fdm_ddpm_step_keyed": (C.c_int, [C.POINTER(DdpmArgs), C.POINTER(NoiseKeys), _vp]),
+    "fdm_window_blend": (C.c_int, [C.POINTER(WindowArgs), _vp]),
     "fdm_advance_cursor": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "fdm_philox_normal": (C.c_int, [_vp, _i64, _i64, _u64, _i64, _i32, _vp]),
     "fdm_vq_quantize": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),
@@ -394,7 +405,9 @@ def self_attention(q, k, v, out, B: int, T: int, t_stride: int, H: int, dh: int,
 
 def ddpm_step(x0_cond, x_t, out, c1, c2, sigma, *, x0_uncond=None, guidance: float = 0.0, noise=None,
               out_bf16=None, t_per_clip=None, t_dev=None, seed: int = 0,
-              clip_index0: int = 0, seed_dev: Optional[torch.Tensor] = None) -> torch.Tensor:
+              clip_index0: int = 0, seed_dev: Optional[torch.Tensor] = None, noise_keys=None) -> torch.Tensor:
+    """noise_keys: None (fdm_ddpm_step), or (clip, e4_offset) int64[B] device tensors or (None, None) (fdm_ddpm_step_keyed:
+    sequence b draws Philox at (clip[b], e4_offset[b] + element))."""
     lib = require_device()
     a = DdpmArgs()
     B = x_t.shape[0]
@@ -411,9 +424,34 @@ def ddpm_step(x0_cond, x_t, out, c1, c2, sigma, *, x0_uncond=None, guidance: flo
     if seed_dev is not None:  # Philox seed read from device memory (int64[1]): replayable graphs, fresh seed per call
         assert seed_dev.dtype == torch.int64 and seed_dev.numel() == 1
     a.seed_dev = _ptr(seed_dev)
-    _check(lib.fdm_ddpm_step(C.byref(a), _stream()))
+    if noise_keys is None:
+        _check(lib.fdm_ddpm_step(C.byref(a), _stream()))
+    else:
+        for k in noise_keys:
+            assert k is None or (k.dtype == torch.int64 and k.is_contiguous() and k.numel() == B)
+        keys = NoiseKeys(_ptr(noise_keys[0]), _ptr(noise_keys[1]))
+        _check(lib.fdm_ddpm_step_keyed(C.byref(a), C.byref(keys), _stream()))
     _launched()
     return out
+
+
+def window_blend(x: torch.Tensor, lam: torch.Tensor, A: int, n_w: int, K: int, S: int, *, x_bf16=None) -> torch.Tensor:
+    """Overlap blend in place (fdm_window_blend): x (A*n_w*K, ...) fp32 holds one window per leading index, window w of
+    clip a and fan-out sequence k at (a*n_w + w)*K + k, each W = S + O rows (O = lam.numel()). Row S + j of window w and row
+    j of window w + 1 both become (1 - lam[j]) * (row S + j) + lam[j] * (row j); x_bf16 gets the bf16 copy."""
+    lib = require_device()
+    n_seq = A * n_w * K
+    O = lam.numel()
+    W = S + O
+    assert x.dtype == torch.float32 and x.is_contiguous() and x.shape[0] == n_seq and x.numel() % (n_seq * W) == 0
+    assert lam.dtype == torch.float32 and lam.is_contiguous()
+    if x_bf16 is not None:
+        assert x_bf16.dtype == torch.bfloat16 and x_bf16.is_contiguous() and x_bf16.numel() == x.numel()
+    a = WindowArgs(_ptr(x), _ptr(x_bf16), _ptr(lam), A, n_w, K, W, S, x.numel() // (n_seq * W))
+    _check(lib.fdm_window_blend(C.byref(a), _stream()))
+    if n_w > 1:
+        _launched()
+    return x
 
 
 def ddim_step(x0_cond, x_t, out, a_recip, a_recipm1, sqrt_an, c, index_dev, *, x0_uncond=None, guidance: float = 0.0,

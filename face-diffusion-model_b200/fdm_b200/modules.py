@@ -19,8 +19,9 @@ from . import lib
 from .audio import AudioEncoderEngine
 from .denoiser import DenoiserEngine, _sin_table
 from .presets import PRESETS, Preset
-from .sampler import SamplerEngine, pool_known
+from .sampler import SamplerEngine, pool_known, pool_windows
 from .vqvae import VQDecoderEngine, quantize
+from .windows import WindowPlan, plan_windows
 
 DEFAULT_PRECISION = os.environ.get("FDM_B200_PRECISION", "bf16")
 
@@ -370,6 +371,7 @@ class GaussianDiffusionBase(nn.Module):
         self.use_cuda_graph = True
         self.__dict__["_last_sampler"] = None
         self.__dict__["_sigma"] = None
+        self.__dict__["_long_audio"] = None
 
     @property
     def last_step_ms(self):
@@ -456,6 +458,105 @@ class GaussianDiffusionBase(nn.Module):
         t0 = int(steps[0])
         return (torch.cat([sa[t0:t0 + 1], ka_mid, torch.ones(1)]), torch.cat([sb[t0:t0 + 1], kb_mid, torch.zeros(1)]))
 
+    def _ddim_schedule(self, n_steps: int):
+        """(t pairs, host tables) of an n_steps DDIM call: the (t, t_next) pairs with t_next >= 0, and per-step coefficients
+        with the reference's own fp32 expressions, evaluated once on the host."""
+        import numpy as np
+        times = list(reversed(np.linspace(-1, 1000 - 1, n_steps + 1).astype(np.int32).tolist()))
+        pairs = [(i, j) for i, j in zip(times[:-1], times[1:]) if j >= 0]
+        t_cur = torch.tensor([p[0] for p in pairs], dtype=torch.long)
+        t_nxt = torch.tensor([p[1] for p in pairs], dtype=torch.long)
+        ac = self.alphas_cumprod.detach().cpu()
+        a, an = ac[t_cur], ac[t_nxt]
+        sigma = 0.0 * torch.sqrt((1 - a) / (1 - an)) * torch.sqrt(1 - a / an)
+        tables = {"a_recip": self.sqrt_recip_alphas_cumprod.detach().cpu()[t_cur],
+                  "a_recipm1": self.sqrt_recipm1_alphas_cumprod.detach().cpu()[t_cur],
+                  "sqrt_an": torch.sqrt(an), "c": torch.sqrt(1 - an - sigma ** 2)}
+        return pairs, tables
+
+    def _check_long(self, P, audio, shape, conds, window, overlap, ddim_steps, steps, step_range, x_T) -> WindowPlan:
+        """The window plan of a sample_long call; every refusal is a ValueError raised before any device state changes."""
+        if not isinstance(audio, torch.Tensor) or audio.dim() != 2 or not audio.is_floating_point():
+            raise ValueError(f"audio must be a floating-point (A, L) tensor, got "
+                             f"{tuple(audio.shape) if isinstance(audio, torch.Tensor) else type(audio).__name__}")
+        if len(conds) != self.n_cond:
+            raise ValueError(f"expected {self.n_cond} condition one-hot(s), got {len(conds)}")
+        plan = plan_windows(P, shape, audio.shape[0], audio.shape[1], window, overlap)
+        B = plan.A * plan.K
+        for c in conds:
+            if not isinstance(c, torch.Tensor) or c.dim() not in (1, 2) or (c.dim() == 2 and c.shape[0] not in (1, B)):
+                raise ValueError(f"a condition has shape {tuple(getattr(c, 'shape', ()))}; the call has {B} sequences "
+                                 f"(give {B} rows or 1)")
+        if ddim_steps is not None:
+            if steps is not None or step_range is not None:
+                raise ValueError("steps / step_range select DDPM steps; give them or ddim_steps, not both")
+            if not isinstance(ddim_steps, int) or isinstance(ddim_steps, bool) or ddim_steps < 2:
+                raise ValueError(f"ddim_steps must be an int >= 2, got {ddim_steps!r}")
+        elif steps is not None and len(steps) == 0:
+            raise ValueError("steps is empty")
+        if x_T is not None and (not isinstance(x_T, torch.Tensor) or not x_T.is_floating_point()
+                                or tuple(x_T.shape) != tuple(shape)):
+            raise ValueError(f"x_T must be a floating-point tensor of the call's shape {tuple(shape)}, got "
+                             f"{tuple(x_T.shape) if isinstance(x_T, torch.Tensor) else type(x_T).__name__}")
+        return plan
+
+    def _window_inputs(self, audio: torch.Tensor, idh, emo, plan: WindowPlan):
+        """(window audio, identity rows, emotion rows) of a windowed call (plan.window_audio / plan.repeat_rows), cached on
+        the identity and version of the inputs and the window layout: a repeat call passes the same tensors on, so the
+        audio encoder's cache, prepare() and the captured graphs are hit."""
+        key = (plan.W, plan.S, plan.n_w, plan.r, plan.K)
+        c = self.__dict__.get("_long_audio")
+        if c is None or c[1] != key or not FDMBase._same(c[0], (audio, idh, emo)):
+            with torch.inference_mode(False):  # normal tensors: the caches downstream read their version counters
+                c = (FDMBase._ident((audio, idh, emo)), key,
+                     (plan.window_audio(audio), plan.repeat_rows(idh), plan.repeat_rows(emo)))
+            self.__dict__["_long_audio"] = c
+        return c[2]
+
+    @torch.inference_mode()
+    def _sample_windows(self, plan: WindowPlan, audio, conds, ddim_steps, steps, step_range, x_T) -> torch.Tensor:
+        """The raw window state (A*n_w*K, fq*W, zdim) after the last step of a windowed sample_long call."""
+        device = self.betas.device
+        idh, emo = self._split(conds)
+        fdm, level, gcond = self._fdm()
+        P = fdm.preset
+        B, z = plan.A * plan.K, P.zdim
+        full = (B, plan.T_pad * P.fq, z)
+
+        def padded(x):  # (B, fq*T, zdim) -> (B, fq*T_pad, zdim), zeros past T
+            out = torch.zeros(full, device=device, dtype=torch.float32)
+            out[:, :plan.T * P.fq] = x.to(device, torch.float32)
+            return out
+
+        ddpm = ddim_steps is None
+        seed = self._call_seed() if ddpm or x_T is None else None
+        # the full-length draw keyed by (seed, clip_index0 + a*K + k): neighbouring windows start identical on their overlap
+        x_full = self._initial_latent(full, device, seed) if x_T is None else padded(x_T)
+        audio_w, idh_w, emo_w = self._window_inputs(audio, idh, emo, plan)
+        eng = fdm.prepare(audio_w, plan.W, idh_w, emo_w, guidance=gcond, fanout=plan.K)
+        sampler = SamplerEngine(eng, self.posterior_mean_coef1, self.posterior_mean_coef2, self._sigma_table(), level)
+        win = pool_windows(eng, plan, self.clip_index0 if ddpm else None)
+        if ddpm:
+            hi, lo = step_range if step_range is not None else self.default_range
+            steps = list(range(hi - 1, lo - 1, -1)) if steps is None else [int(t) for t in steps]
+            noise = self.noise_source
+            if callable(noise):  # full-length host noise, gathered into windows like x_T
+                noise = (lambda t, src=noise: plan.gather(padded(src(t))))
+            tail = self._tail(fdm, audio_w, plan.W, idh_w, emo_w, gcond, len(steps), plan.K)
+            with lib.nvtx_range("sampling_loop"):
+                out = sampler.run(plan.gather(x_full), steps, noise=noise, seed=seed, clip_index0=self.clip_index0,
+                                  graph=self.use_cuda_graph, time_steps=getattr(self, "time_steps", False), tail=tail,
+                                  windows=win)
+        else:
+            pairs, tables = self._ddim_schedule(ddim_steps)
+            tables = {k: v.to(device=device, dtype=torch.float32).contiguous() for k, v in tables.items()}
+            tail = self._tail(fdm, audio_w, plan.W, idh_w, emo_w, gcond, len(pairs), plan.K)
+            with lib.nvtx_range("ddim_loop"):
+                out = sampler.run(plan.gather(x_full), [p[0] for p in pairs], graph=self.use_cuda_graph, ddim=tables,
+                                  time_steps=getattr(self, "time_steps", False), tail=tail, windows=win)
+        self.__dict__["_last_sampler"] = sampler
+        return out
+
     # -- reference API ----------------------------------------------------------------------------------
     @torch.inference_mode()
     def p_sample(self, x, t, audio, *conds, clip_denoised=False, noise=None):
@@ -504,7 +605,6 @@ class GaussianDiffusionBase(nn.Module):
         """Deterministic DDIM sampling, eta = 0 (reference diffusion_BIWI_encoder_decoder.py:675-710):
         ddim_sample(audio, shape, id_one_hot, steps=500). The reference's last time pair (t, -1) evaluates the
         denoiser and then leaves the sample unchanged; that evaluation is skipped here."""
-        import numpy as np
         n_c = self.n_cond
         conds = conds_and_steps[:n_c]
         n_steps = conds_and_steps[n_c] if len(conds_and_steps) > n_c else 500
@@ -514,17 +614,7 @@ class GaussianDiffusionBase(nn.Module):
         P = fdm.preset
         shape = tuple(latent_motion_shape)
         kn = self._check_known(shape, P, known, known_mask)
-        times = list(reversed(np.linspace(-1, 1000 - 1, n_steps + 1).astype(np.int32).tolist()))
-        pairs = [(i, j) for i, j in zip(times[:-1], times[1:]) if j >= 0]
-        t_cur = torch.tensor([p[0] for p in pairs], dtype=torch.long)
-        t_nxt = torch.tensor([p[1] for p in pairs], dtype=torch.long)
-        # per-step coefficients with the reference's own fp32 expressions, evaluated once on the host
-        ac = self.alphas_cumprod.detach().cpu()
-        a, an = ac[t_cur], ac[t_nxt]
-        sigma = 0.0 * torch.sqrt((1 - a) / (1 - an)) * torch.sqrt(1 - a / an)
-        tables = {"a_recip": self.sqrt_recip_alphas_cumprod.detach().cpu()[t_cur],
-                  "a_recipm1": self.sqrt_recipm1_alphas_cumprod.detach().cpu()[t_cur],
-                  "sqrt_an": torch.sqrt(an), "c": torch.sqrt(1 - an - sigma ** 2)}
+        pairs, tables = self._ddim_schedule(n_steps)
         known_ab = None if kn is None else self._known_tables([p[0] for p in pairs], tables)
         tables = {k: v.to(device=device, dtype=torch.float32).contiguous() for k, v in tables.items()}
         seed = self._call_seed() if x_T is None or kn is not None else None
@@ -545,6 +635,35 @@ class GaussianDiffusionBase(nn.Module):
     @torch.inference_mode()
     def sample(self, audio, latent_motion_shape, *conds, **kw):
         return self.p_sample_loop(latent_motion_shape, audio, *conds, **kw)
+
+    @torch.inference_mode()
+    def sample_long(self, audio, latent_motion_shape, *conds, window: Optional[int] = None, overlap: Optional[int] = None,
+                    ddim_steps: Optional[int] = None, steps: Optional[Sequence[int]] = None,
+                    step_range: Optional[Sequence[int]] = None, x_T: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Sample audio of any length in one call: (A, L) audio, latent shape (B, fq*T, zdim) with B = A*K (fan-out as in
+        sample) -> (B, fq*T, zdim) float32, the layout sample() returns, for quant / decode.
+
+        The T frames are cut into windows of `window` frames (default 14 periods: 420 for VOCASET / MEAD, 350 for BIWI)
+        that share `overlap` frames with their neighbours (default 2 periods). Window w covers frames [w*S, w*S + window),
+        S = window - overlap, and its audio is encoded as its own clip. All windows of all clips are sampled as one batch,
+        and after every step each shared frame's two rows are replaced by (1 - l_j) * earlier window + l_j * later window,
+        l_j = (j + 1) / (overlap + 1) at overlap row j. DDPM draws its noise per absolute frame (Philox keyed by the long
+        sequence's global index clip_index0 + a*K + k and the frame), so both windows of a frame add the same noise.
+        x_T (default: the Philox draw sample() would make for the full length) is gathered into the windows.
+
+        ddim_steps None: DDPM over `steps` / `step_range` as in p_sample_loop (default: the preset's range); an int: DDIM
+        with that many steps, as in ddim_sample. With T <= window the call is sample() / ddim_sample() of the same arguments.
+        Refused with ValueError, before anything runs: overlap outside [1, window // 2], window - overlap not a multiple of
+        the preset's period, window > 600, audio yielding fewer than T frames, and wrong shapes, row counts or dtypes.
+        Known frames (known= / known_mask=) and tap= are not accepted here."""
+        fdm, _, _ = self._fdm()
+        shape = tuple(int(s) for s in latent_motion_shape)
+        plan = self._check_long(fdm.preset, audio, shape, conds, window, overlap, ddim_steps, steps, step_range, x_T)
+        if plan.n_w == 1:
+            if ddim_steps is None:
+                return self.p_sample_loop(shape, audio, *conds, x_T=x_T, step_range=step_range, steps=steps)
+            return self.ddim_sample(audio, shape, *conds, ddim_steps, x_T=x_T)
+        return plan.assemble(self._sample_windows(plan, audio, conds, ddim_steps, steps, step_range, x_T))
 
 
 # ---------------------------------------------------------------------------------------------------

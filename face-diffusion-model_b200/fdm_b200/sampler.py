@@ -43,6 +43,30 @@ def pool_known(den: DenoiserEngine, latent: torch.Tensor, mask: torch.Tensor, ka
     return KnownFrames(lat, m, kab[0], kab[1])
 
 
+class Windows(NamedTuple):
+    """Overlapping windows of a long-audio call (fdm_b200.windows.WindowPlan) in pooled buffers of the denoiser engine
+    (stable addresses: a new call of the same layout replays the cached step graphs). After every step's update,
+    fdm_window_blend mixes the overlap rows; DDPM draws its noise with the per-window keys (fdm_ddpm_step_keyed)."""
+    lam: torch.Tensor                    # (O,) fp32 blend weights
+    keys: Optional[tuple]                # (clip, e4_offset) int64 per window sequence, or None (DDIM: no draws)
+    A: int
+    n_w: int
+    K: int
+    S: int
+
+
+def pool_windows(den: DenoiserEngine, plan, clip_index0: Optional[int]) -> Windows:
+    """Copy a plan's blend weights and, unless clip_index0 is None, its noise keys into the engine's pooled buffers."""
+    lam = den.buf("smp_win_lambda", (plan.O,), torch.float32)
+    lam.copy_(plan.weights())
+    keys = None
+    if clip_index0 is not None:
+        kb = den.buf("smp_win_keys", (2, plan.n_seq), torch.int64)
+        kb.copy_(torch.stack(plan.noise_keys(clip_index0, den.P.d)))
+        keys = (kb[0], kb[1])
+    return Windows(lam, keys, plan.A, plan.n_w, plan.K, plan.S)
+
+
 class SamplerEngine:
     def __init__(self, denoiser: DenoiserEngine, c1: torch.Tensor, c2: torch.Tensor, sigma: torch.Tensor,
                  guidance_level: Optional[float] = None):
@@ -68,7 +92,7 @@ class SamplerEngine:
     def run(self, x_T: torch.Tensor, steps: Sequence[int], noise: NoiseSpec = "philox", seed: int = 0,
             clip_index0: int = 0, graph: bool = True, tap: Optional[Callable[[int, torch.Tensor], None]] = None,
             time_steps: bool = False, ddim: Optional[dict] = None, tail=None,
-            known: Optional[KnownFrames] = None) -> torch.Tensor:
+            known: Optional[KnownFrames] = None, windows: Optional[Windows] = None) -> torch.Tensor:
         """x_T (B, fq*T, zdim) fp32 on device; steps: the t values in execution order (e.g. 999..0).
         noise: "philox" (in-kernel counter-based generator), or a callable t -> tensor (host- or device-side,
         same shape as x_T) that is copied in before every step with t > 0 (parity runs).
@@ -80,7 +104,10 @@ class SamplerEngine:
         known: None, or KnownFrames (pool_known): the start state and the state after every step are replaced on the known
         rows (one fdm_known_frames launch after each step's update). Its z is the draw the update used at that element:
         the host noise buffer, or Philox at (seed, clip_index0 + b, t); after the last step the known rows hold
-        `known.latent` bit for bit."""
+        `known.latent` bit for bit.
+        windows: None, or Windows (pool_windows): the B sequences are the windows of a long-audio call; every step's update
+        (graph-replayed or high-precision tail) is followed by one fdm_window_blend launch, and DDPM keys its Philox draw
+        by long sequence and absolute frame (windows.keys)."""
         den = self.den
         B, T, d, S = den.B, den.T, den.P.d, den.passes
         assert x_T.is_cuda and x_T.dtype == torch.float32 and x_T.numel() == B * T * d, "x_T does not match prepare()"
@@ -106,6 +133,8 @@ class SamplerEngine:
         assert host_noise or ddim is not None or noise in (None, "philox")
         if known is not None:
             assert known.latent.shape == x.shape and known.mask.numel() == B * T and known.ka.numel() == len(steps) + 1
+        if windows is not None:
+            assert B == windows.A * windows.n_w * windows.K and T == windows.S + windows.lam.numel()
 
         def replace_known(offset: int, z=None):
             lib.known_frames(x, known.latent, known.mask, known.ka, known.kb, cursor, offset=offset, noise=z, x_bf16=xin_bf,
@@ -116,13 +145,15 @@ class SamplerEngine:
             if ddim is None:
                 lib.ddpm_step(x0[0], x, x, self.c1, self.c2, self.sigma, x0_uncond=x0[1] if S == 2 else None,
                               guidance=float(self.level) if S == 2 else 0.0, noise=noise_buf, out_bf16=xin_bf, t_dev=t_dev,
-                              seed_dev=seed_dev, clip_index0=clip_index0)
+                              seed_dev=seed_dev, clip_index0=clip_index0, noise_keys=None if windows is None else windows.keys)
             else:
                 lib.ddim_step(x0[0], x, x, ddim["a_recip"], ddim["a_recipm1"], ddim["sqrt_an"], ddim["c"], cursor,
                               x0_uncond=x0[1] if S == 2 else None, guidance=float(self.level) if S == 2 else 0.0,
                               out_bf16=xin_bf)
             if known is not None:  # state after step `cursor`: table entry cursor + 1
                 replace_known(1, noise_buf)
+            if windows is not None:
+                lib.window_blend(x, windows.lam, windows.A, windows.n_w, windows.K, windows.S, x_bf16=xin_bf)
             lib.advance_cursor(cursor, sched, t_dev)
 
         def reset():
@@ -163,6 +194,9 @@ class SamplerEngine:
                    tuple(a.data_ptr() for a in den.addend))
             if known is not None:
                 key += (known.latent.data_ptr(), known.mask.data_ptr(), known.ka.data_ptr(), known.kb.data_ptr())
+            if windows is not None:
+                key += (windows.lam.data_ptr(), windows.A, windows.n_w, windows.K, windows.S,
+                        None if windows.keys is None else tuple(k.data_ptr() for k in windows.keys))
             hit = den.graph_cache.get(key)
             if hit is None:
                 reset()

@@ -229,6 +229,30 @@ typedef struct fdm_known_args {
 } fdm_known_args;
 int fdm_known_frames(const fdm_known_args* args, void* stream);
 
+/* Noise keys of a windowed (long-audio) sampling call: fdm_ddpm_step with the Philox normal of sequence b drawn at
+ *   clip = clip[b], element = e4_offset[b] + e0        (e0: float4 index within the sequence)
+ * instead of (clip_index0 + b, e0). Window w of long sequence g gets clip = clip_index0 + g and e4_offset = w*S*d/4 (S: window
+ * stride in frames, d: elements per frame), so every window that covers an absolute frame draws the same z for it.
+ * keys == NULL, or both pointers NULL, is fdm_ddpm_step. Device arrays of B entries, written before the step is launched. */
+typedef struct fdm_noise_keys {
+  const int64_t* clip; const int64_t* e4_offset;
+} fdm_noise_keys;
+int fdm_ddpm_step_keyed(const fdm_ddpm_args* args, const fdm_noise_keys* keys, void* stream);
+
+/* Overlap blend of a windowed sampling call, in place. The state holds A audio clips x n_w windows x K sequences per clip,
+ * window sequence (a*n_w + w)*K + k, W rows of d elements each; window w + 1 starts S rows after window w, so rows [S, W) of
+ * window w and rows [0, O) of window w + 1 (O = W - S) are the same frames. For every such pair (a, w < n_w - 1, k, j < O):
+ *   o = (1 - lambda[j]) * x_lo + lambda[j] * x_hi      (each product rounded, then added)
+ *   x_lo = row S + j of window w, x_hi = row j of window w + 1; o is written to both rows (and to x_bf16, when given).
+ * lambda: O fp32 weights in device memory. Rows outside overlaps are not touched; n_w == 1 launches nothing. */
+typedef struct fdm_window_args {
+  float* x; void* x_bf16;
+  const float* lambda;
+  int64_t A; int64_t n_w; int64_t K;   /* audio clips, windows per clip, sequences per clip */
+  int64_t W; int64_t S; int64_t d;     /* rows per window, window stride in rows, elements per row */
+} fdm_window_args;
+int fdm_window_blend(const fdm_window_args* args, void* stream);
+
 /* End of a graph-replayed step: cursor[0] += 1; t_dev[0] = t_sched[min(cursor[0], n_sched-1)]. */
 int fdm_advance_cursor(int32_t* cursor_dev, const int32_t* t_sched, int32_t n_sched, int32_t* t_dev, void* stream);
 /* Fill out[B*elems_per_clip] with the same Philox normals the fused step would draw for step t. */
