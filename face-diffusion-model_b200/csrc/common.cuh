@@ -35,6 +35,10 @@ int fdm_gemm_init_device();
 int fdm_sm_count();  // cached multiprocessor count of the current device
 bool fdm_pdl_enabled();  // programmatic dependent launch for the hot-loop kernels (on by default; env FDM_B200_PDL=0 turns it off)
 
+// One tile of a VQ kernel with per-row codebook slices (fdm_vq_quantize_runs): rows [l0, l0 + nrows) of clip b, codebook
+// slice offset `off`. vq.cu cuts the run table into these per call (no tile crosses a run); the kernels read one per tile.
+struct alignas(16) VqTile { int b, l0, nrows, off; };
+
 // ---- programmatic dependent launch (PDL) -------------------------------------------------------
 // Hot-loop kernels are launched with programmaticStreamSerialization: kernel N+1 may be scheduled while kernel N
 // drains, runs its prologue (barrier init, TMEM alloc, descriptor prefetch, index math) and then blocks in

@@ -321,10 +321,27 @@ __global__ void __launch_bounds__(256) resample_poly_kernel(const float* __restr
 // the perplexity. One pass over z and the indices (the winning code rows come from the L2-resident codebook) instead of
 // torch's three passes over (rows, D) temporaries. One warp per row; per-block partial sums in a fixed order (the host adds
 // the `gridDim.x` partials), integer atomics for the histogram: deterministic.
+// Codebook offset of a row: per clip (code_offset), from the run table (runs.clip_run != NULL: the last run of the row's clip that
+// starts at or before it, by bisection), or 0.
+__device__ __forceinline__ int64_t row_slice(const int64_t* __restrict__ code_offset, const fdm_vq_runs& runs, int64_t row,
+                                             int64_t L) {
+  const int64_t b = row / L;
+  if (runs.clip_run) {
+    const int64_t l = row - b * L;
+    int64_t lo = runs.clip_run[b], hi = runs.clip_run[b + 1] - 1;
+    while (lo < hi) {
+      const int64_t mid = (lo + hi + 1) >> 1;
+      if (runs.run_l0[mid] <= l) lo = mid; else hi = mid - 1;
+    }
+    return runs.run_offset[lo];
+  }
+  return code_offset ? code_offset[b] : 0;
+}
+
 __global__ void __launch_bounds__(256) vq_stats_kernel(const float* __restrict__ z, const float* __restrict__ codebook,
                                                        const int64_t* __restrict__ code_offset, const int64_t* __restrict__ indices,
                                                        int64_t rows, int64_t L, int D, int n_codes, float* __restrict__ partials,
-                                                       unsigned long long* __restrict__ hist) {
+                                                       unsigned long long* __restrict__ hist, const fdm_vq_runs runs) {
   extern __shared__ unsigned int sh_hist[];  // n_codes counters, then 8 floats
   float* red = reinterpret_cast<float*>(sh_hist + n_codes);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -347,7 +364,7 @@ __global__ void __launch_bounds__(256) vq_stats_kernel(const float* __restrict__
 #pragma unroll
       for (int q = 0; q < RW; ++q) {
         if (idx[q] < 0) continue;
-        const int64_t off = code_offset ? code_offset[(row0 + q) / L] : 0;
+        const int64_t off = row_slice(code_offset, runs, row0 + q, L);
         const float2 e = __ldg(reinterpret_cast<const float2*>(codebook + (off + idx[q]) * 64) + lane);
         const float d0 = e.x - a[q].x, d1 = e.y - a[q].y;
         acc = fmaf(d0, d0, acc);
@@ -357,7 +374,7 @@ __global__ void __launch_bounds__(256) vq_stats_kernel(const float* __restrict__
     } else {
       for (int q = 0; q < RW && row0 + q < rows; ++q) {
         const int64_t row = row0 + q, id = indices[row];
-        const int64_t off = code_offset ? code_offset[row / L] : 0;
+        const int64_t off = row_slice(code_offset, runs, row, L);
         const float* zr = z + row * D;
         const float* er = codebook + (off + id) * D;
         for (int k = lane; k < D; k += 32) {
@@ -527,7 +544,23 @@ extern "C" int fdm_vq_stats(const float* z, const float* codebook, const int64_t
   const size_t smem = static_cast<size_t>(n_codes) * 4 + 32;
   vq_stats_kernel<<<static_cast<unsigned>(n_partials), 256, smem, reinterpret_cast<cudaStream_t>(stream)>>>(
       z, codebook, code_offset, indices, B * L, L, static_cast<int>(D), static_cast<int>(n_codes), sqerr_partials,
-      reinterpret_cast<unsigned long long*>(hist));
+      reinterpret_cast<unsigned long long*>(hist), fdm_vq_runs{nullptr, nullptr, nullptr, 0});
+  FDM_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int fdm_vq_stats_runs(const float* z, const float* codebook, const fdm_vq_runs* runs, const int64_t* indices,
+                                 int64_t B, int64_t L, int64_t D, int64_t n_codes, float* sqerr_partials, int64_t n_partials,
+                                 int64_t* hist, void* stream) {
+  FDM_CHECK_ARG(z && codebook && indices && sqerr_partials && hist && B > 0 && L > 0 && D > 0 && D <= 1024 && n_codes > 0 &&
+                    n_codes <= 8192 && n_partials > 0 && n_partials <= 65535,
+                "fdm_vq_stats_runs: bad arguments");
+  FDM_CHECK_ARG(runs && runs->clip_run && runs->run_l0 && runs->run_offset && runs->n_runs >= B,
+                "fdm_vq_stats_runs: the run table needs clip_run, run_l0, run_offset and at least one run per clip");
+  const size_t smem = static_cast<size_t>(n_codes) * 4 + 32;
+  vq_stats_kernel<<<static_cast<unsigned>(n_partials), 256, smem, reinterpret_cast<cudaStream_t>(stream)>>>(
+      z, codebook, nullptr, indices, B * L, L, static_cast<int>(D), static_cast<int>(n_codes), sqerr_partials,
+      reinterpret_cast<unsigned long long*>(hist), *runs);
   FDM_CHECK_LAUNCH();
   return 0;
 }

@@ -25,11 +25,13 @@
 
 int fdm_vq_tc_launch(const float* z, const float* codebook, const int64_t* code_offset, int64_t B, int64_t L, int64_t D,
                      int n_codes, int64_t* indices, float* zq_bdl, float* zq_rows, unsigned long long* recheck_rows,
-                     float* dbg_acc, cudaStream_t stream) {
+                     float* dbg_acc, const VqTile* tiles, const int* tile_count, int64_t max_tiles, cudaStream_t stream) {
   if (D == 64)
-    return vq_tc64::launch(z, codebook, code_offset, B, L, n_codes, indices, zq_bdl, zq_rows, recheck_rows, dbg_acc, stream);
+    return vq_tc64::launch(z, codebook, code_offset, B, L, n_codes, indices, zq_bdl, zq_rows, recheck_rows, dbg_acc, tiles,
+                           tile_count, max_tiles, stream);
   if (D == 128)
-    return vq_tc128::launch(z, codebook, code_offset, B, L, n_codes, indices, zq_bdl, zq_rows, recheck_rows, dbg_acc, stream);
+    return vq_tc128::launch(z, codebook, code_offset, B, L, n_codes, indices, zq_bdl, zq_rows, recheck_rows, dbg_acc, tiles,
+                            tile_count, max_tiles, stream);
   FDM_CHECK_ARG(false, "fdm_vq_quantize: the tensor-core path needs D = 64 or 128 (got %lld)", (long long)D);
   return 0;
 }

@@ -35,7 +35,9 @@
 //   warp 9      13 x tcgen05.mma (128 x 256 x 16) per tile into one of two 256-column TMEM accumulators
 //   warps 0-7   two epilogue groups (one per accumulator): tcgen05.ld, pass A / pass B over the scores, recheck,
 //               int64 index, gather of the winning code row into z_q (B, D, L) and / or (B, L, D)
-// Per-clip codebook slices (MEAD emotions) are handled as segments: the CTA drains, reloads the slice, continues.
+// Per-clip codebook slices (MEAD emotions) are handled as segments: the CTA drains, reloads the slice, continues. Per-row
+// slices (fdm_vq_quantize_runs) come as a table of tiles that never cross a run, so a segment is a stretch of tiles of runs with
+// one slice; a run's last tile may be partial and is handled like a clip's ragged last tile.
 // This file is the kernel body; vq_tc.cu includes it once per latent width (VQ_D = 64, 128; VQ_NS = its namespace).
 // D = 128 (BIWI, models/utils/config.py:44-60 / models/vq_vae.py:219-248): a 128-row tile is processed as KH = 2
 // K-HALVES of 64 dimensions. Each half is one A-operand stage (hi, lo; the same 32 KB the D = 64 kernel uses per tile)
@@ -201,9 +203,25 @@ struct Params {
   unsigned long long* recheck_rows;  // optional counter of rows that took the exact path
   float* dbg_acc;                    // optional [rows, n_codes] dump of a_j = dot_j - ee_j / 2 from the tensor cores (tests)
   int tiles_per_clip, num_tiles;  // 32-bit on purpose: tile -> (clip, row) divisions stay inline
+  const VqTile* tiles;            // per-row slices (fdm_vq_quantize_runs): tile t is tiles[t], *tile_count of them; else NULL
+  const int* tile_count;
   float window_scale;  // 1.0; profiling knob FDM_B200_VQ_WINDOW (0 = never take the exact pass: NOT bit-exact)
   int l2_ahead;        // tiles prefetched into L2 ahead of the shared-memory ring (FDM_B200_VQ_L2_AHEAD, default L2_AHEAD)
 };
+
+// Clip, first row and row count of tile tl: 128-row tiles of whole clips, or (TL: fdm_vq_quantize_runs) the caller's tile table,
+// one 16-byte load per tile. The kernel is instantiated for both, so the per-clip path compiles exactly as without tables.
+struct TileRef { int b; int64_t l0; int nrows; };
+template <bool TL>
+__device__ __forceinline__ TileRef tile_ref(const VqTile* tiles, int tpc, int64_t L, int tl) {
+  if constexpr (TL) {
+    const int4 t = __ldg(reinterpret_cast<const int4*>(tiles) + tl);
+    return TileRef{t.x, t.y, t.z};
+  }
+  const int b = tl / tpc;
+  const int64_t l0 = static_cast<int64_t>(tl - b * tpc) * TILE_ROWS;
+  return TileRef{b, l0, static_cast<int>(min(static_cast<int64_t>(TILE_ROWS), L - l0))};
+}
 
 // Exact pass for ONE flagged row (rare, latency-bound; out of line and lean on registers: with 226 KB of the SM's
 // 256 KB carved out as shared memory every local-memory spill is an L2 round trip, and an earlier version that kept 16
@@ -271,16 +289,22 @@ struct Ctx {
 
 // A segment is a maximal run of this CTA's tiles that share one codebook slice. All threads call this at the start
 // of every segment: they drain (barrier), convert the slice into the B operands, compute ee, and return its end.
+template <bool TL>
 __device__ __noinline__ int segment_begin(const Params& p, const Ctx& cx, int tile, int64_t* off_out) {
   const int tid = threadIdx.x;
   const int n_codes = p.n_codes, tpc = p.tiles_per_clip;
   const uint32_t base = cx.base;
   float* ee = reinterpret_cast<float*>(cx.smem + OFF_EE);
   uint32_t* ee_max_bits = reinterpret_cast<uint32_t*>(cx.smem + OFF_MISC + 4);
-  const int b0 = tile / tpc;
-  const int64_t off = p.code_offset ? p.code_offset[b0] : 0;
+  int64_t off = 0;
   int seg_end = cx.t_end;
-  if (p.code_offset) {
+  if constexpr (TL) {  // (a run's tiles are consecutive, so a slice change between tiles is a run boundary)
+    off = p.tiles[tile].off;
+    for (int t = tile + 1; t < cx.t_end; ++t)
+      if (p.tiles[t].off != off) { seg_end = t; break; }
+  } else if (p.code_offset) {
+    const int b0 = tile / tpc;
+    off = p.code_offset[b0];
     for (int bb = b0 + 1; bb * tpc < cx.t_end; ++bb)
       if (p.code_offset[bb] != off) { seg_end = bb * tpc; break; }
   }
@@ -323,10 +347,12 @@ __device__ __noinline__ int segment_begin(const Params& p, const Ctx& cx, int ti
 }
 
 // ===== converters (warps 10-13): staged fp32 rows -> bf16 (hi, lo) A operand + |z|^2 estimate =====
+template <bool TL>
 __device__ __noinline__ void role_convert(const Params& p, const Ctx& cx) {
   const int tid = threadIdx.x - CONV_WARP0 * 32, lane = tid & 31;
   const int64_t L = p.L;
   const int tpc = p.tiles_per_clip;
+  const VqTile* const tiles = p.tiles;
   const uint32_t base = cx.base;
   // (Params / Ctx live in memory behind references: everything the loops need is copied into registers first)
   uint8_t* const smem = cx.smem;
@@ -336,10 +362,9 @@ __device__ __noinline__ void role_convert(const Params& p, const Ctx& cx) {
   const int row_q = tid >> 3, c8 = tid & 7;  // this thread's (row, 8-float column block) inside a 16-row slab
   // (D = 128) address of this thread's unit 0 (row row_q, columns 64 h + 8 c8 ..) of sub-tile (tile, K-half), rows in the tile
   auto unit0_of = [&](int tl2, int h2, int& nrows2) -> const float* {
-    const int b2 = tl2 / tpc;
-    const int64_t l2 = static_cast<int64_t>(tl2 - b2 * tpc) * TILE_ROWS;
-    nrows2 = static_cast<int>(min(static_cast<int64_t>(TILE_ROWS), L - l2));
-    return p.z + (static_cast<int64_t>(b2) * L + l2 + row_q) * D + h2 * 64 + c8 * 8;
+    const TileRef t2 = tile_ref<TL>(tiles, tpc, L, tl2);
+    nrows2 = t2.nrows;
+    return p.z + (static_cast<int64_t>(t2.b) * L + t2.l0 + row_q) * D + h2 * 64 + c8 * 8;
   };
   float4 x0[CONV_UNITS], x1[CONV_UNITS];
   if (!RING && cx.t_begin < t_end) {  // the first sub-tile's loads
@@ -359,11 +384,9 @@ __device__ __noinline__ void role_convert(const Params& p, const Ctx& cx) {
   }
   for (int tile = cx.t_begin; tile < t_end;) {
     int64_t off;
-    const int seg_end = segment_begin(p, cx, tile, &off);
+    const int seg_end = segment_begin<TL>(p, cx, tile, &off);
     for (int tl = tile; tl < seg_end; ++tl, ++it) {
-      const int b = tl / tpc;
-      const int64_t l0 = static_cast<int64_t>(tl - b * tpc) * TILE_ROWS;
-      const int nrows = static_cast<int>(min(static_cast<int64_t>(TILE_ROWS), L - l0));
+      const int nrows = RING ? tile_ref<TL>(tiles, tpc, L, tl).nrows : 0;  // (the no-ring path takes row counts from unit0_of)
       float* zz = zzs + (it & (ZZ_SLOTS - 1)) * TILE_ROWS;
       if (RING) {
         const int as = it & 1;
@@ -435,10 +458,8 @@ __device__ __noinline__ void role_convert(const Params& p, const Ctx& cx) {
           const int ahead = p.l2_ahead;
           const int first = (tl == cx.t_begin) ? tl + 1 : tl + ahead;
           for (int ta = first; ta <= tl + ahead && ta < t_end; ++ta) {
-            const int ba = ta / tpc;
-            const int64_t la = static_cast<int64_t>(ta - ba * tpc) * TILE_ROWS;
-            const int na = static_cast<int>(min(static_cast<int64_t>(TILE_ROWS), L - la));
-            bulk_prefetch_l2(p.z + (static_cast<int64_t>(ba) * L + la) * D, static_cast<uint32_t>(na) * D * 4);
+            const TileRef a = tile_ref<TL>(tiles, tpc, L, ta);
+            bulk_prefetch_l2(p.z + (static_cast<int64_t>(a.b) * L + a.l0) * D, static_cast<uint32_t>(a.nrows) * D * 4);
           }
         }
 #pragma unroll 1
@@ -498,6 +519,7 @@ __device__ __noinline__ void role_convert(const Params& p, const Ctx& cx) {
 }
 
 // ===== MMA issuer (warp 9) =====
+template <bool TL>
 __device__ __noinline__ void role_mma(const Params& p, const Ctx& cx) {
   const int lane = threadIdx.x & 31;
   const uint32_t base = cx.base;
@@ -510,7 +532,7 @@ __device__ __noinline__ void role_mma(const Params& p, const Ctx& cx) {
   uint32_t it = 0;
   for (int tile = cx.t_begin; tile < t_end;) {
     int64_t off;
-    const int seg_end = segment_begin(p, cx, tile, &off);
+    const int seg_end = segment_begin<TL>(p, cx, tile, &off);
     for (int tl = tile; tl < seg_end; ++tl, ++it) {
       if (lane == 0) {
         const int acc = it & 1;
@@ -549,31 +571,32 @@ __device__ __noinline__ void role_mma(const Params& p, const Ctx& cx) {
 }
 
 // ===== loader (warp 8): 1-D bulk copies of contiguous fp32 rows =====
+template <bool TL>
 __device__ __noinline__ void role_load(const Params& p, const Ctx& cx) {
   const int lane = threadIdx.x & 31;
   const int64_t L = p.L;
   const int tpc = p.tiles_per_clip;
   const uint32_t base = cx.base;
   const float* const zsrc = p.z;
+  const VqTile* const tiles = p.tiles;
   const int t_end = cx.t_end;
   uint32_t it = 0, hc = 0;
   for (int tile = cx.t_begin; tile < t_end;) {
     int64_t off;
-    const int seg_end = segment_begin(p, cx, tile, &off);
+    const int seg_end = segment_begin<TL>(p, cx, tile, &off);
     for (int tl = tile; RING && tl < seg_end; ++tl, ++it) {  // (D = 128: the converters load; this warp only takes part in the segment barriers)
-      const int b = tl / tpc;
-      const int64_t l0 = static_cast<int64_t>(tl - b * tpc) * TILE_ROWS;
-      const int nrows = static_cast<int>(min(static_cast<int64_t>(TILE_ROWS), L - l0));
+      const TileRef t0 = tile_ref<TL>(tiles, tpc, L, tl);
+      const int b = t0.b;
+      const int64_t l0 = t0.l0;
+      const int nrows = t0.nrows;
       // The ring holds 2.25 tiles = 72 KB, which at ~1.8 us of loaded HBM latency is ~40 GB/s per SM: latency-bound at
       // a third of the HBM rate. Tiles further ahead are pulled into L2 so that the ring's copies are L2 hits.
       if (lane == 0) {
         const int ahead = p.l2_ahead;
         const int first = (tl == cx.t_begin) ? tl + 1 : tl + ahead;
         for (int ta = first; ta <= tl + ahead && ta < t_end; ++ta) {
-          const int ba = ta / tpc;
-          const int64_t la = static_cast<int64_t>(ta - ba * tpc) * TILE_ROWS;
-          const int na = static_cast<int>(min(static_cast<int64_t>(TILE_ROWS), L - la));
-          bulk_prefetch_l2(zsrc + (static_cast<int64_t>(ba) * L + la) * D, static_cast<uint32_t>(na) * D * 4);
+          const TileRef a = tile_ref<TL>(tiles, tpc, L, ta);
+          bulk_prefetch_l2(zsrc + (static_cast<int64_t>(a.b) * L + a.l0) * D, static_cast<uint32_t>(a.nrows) * D * 4);
         }
       }
       for (int part = 0; part < TILE_ROWS / STG_ROWS; ++part) {
@@ -646,6 +669,7 @@ __device__ __noinline__ void drain_deferred(const Params& p, const Ctx& cx, cons
 }
 
 // ===== epilogue (warps 0-7): group g owns accumulator g =====
+template <bool TL>
 __device__ __noinline__ void role_epilogue(const Params& p, const Ctx& cx) {
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int n_codes = p.n_codes, nchunks = n_codes >> 5;
@@ -671,15 +695,16 @@ __device__ __noinline__ void role_epilogue(const Params& p, const Ctx& cx) {
   uint32_t it = 0;
   for (int tile = cx.t_begin; tile < t_end;) {
     int64_t off;
-    const int seg_end = segment_begin(p, cx, tile, &off);
+    const int seg_end = segment_begin<TL>(p, cx, tile, &off);
     const float* cbg = codebook + off * D;
     const float ee_max = __uint_as_float(*reinterpret_cast<const uint32_t*>(smem + OFF_MISC + 4));
     const float se_max = sqrtf(ee_max) * 1.001f;
     for (int tl = tile; tl < seg_end; ++tl, ++it) {
       if ((it & 1) != static_cast<uint32_t>(grp)) continue;
-      const int64_t b = tl / tpc;
-      const int64_t l0 = static_cast<int64_t>(tl - static_cast<int>(b) * tpc) * TILE_ROWS;
-      const int nrows = static_cast<int>(min(static_cast<int64_t>(TILE_ROWS), L - l0));
+      const TileRef t0 = tile_ref<TL>(p.tiles, tpc, L, tl);
+      const int64_t b = t0.b;
+      const int64_t l0 = t0.l0;
+      const int nrows = t0.nrows;
       const bool row_ok = row < nrows;
       const int64_t grow = b * L + l0 + row;
       if (quad == 0) TRACE(7);
@@ -900,6 +925,7 @@ __device__ __noinline__ void role_epilogue(const Params& p, const Ctx& cx) {
   }
 }
 
+template <bool TL>
 __global__ void __launch_bounds__(NUM_THREADS, 1) vq_tc_kernel(const __grid_constant__ Params p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = smem_u32(smem_raw);
@@ -928,25 +954,28 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) vq_tc_kernel(const __grid_cons
   __syncthreads();
   tcgen05_fence_after();
   cx.tmem_base = *tmem_slot;
-  cx.t_begin = static_cast<int>(static_cast<uint64_t>(blockIdx.x) * static_cast<uint32_t>(p.num_tiles) / gridDim.x);
-  cx.t_end = static_cast<int>(static_cast<uint64_t>(blockIdx.x + 1) * static_cast<uint32_t>(p.num_tiles) / gridDim.x);
+  const uint32_t num_tiles = static_cast<uint32_t>(TL ? *p.tile_count : p.num_tiles);
+  cx.t_begin = static_cast<int>(static_cast<uint64_t>(blockIdx.x) * num_tiles / gridDim.x);
+  cx.t_end = static_cast<int>(static_cast<uint64_t>(blockIdx.x + 1) * num_tiles / gridDim.x);
 
-  if (warp >= CONV_WARP0) role_convert(p, cx);
-  else if (warp == MMA_WARP) role_mma(p, cx);
-  else if (warp == LOAD_WARP) role_load(p, cx);
-  else role_epilogue(p, cx);
+  if (warp >= CONV_WARP0) role_convert<TL>(p, cx);
+  else if (warp == MMA_WARP) role_mma<TL>(p, cx);
+  else if (warp == LOAD_WARP) role_load<TL>(p, cx);
+  else role_epilogue<TL>(p, cx);
 
   tcgen05_fence_before();
   __syncthreads();
   if (warp == MMA_WARP) tmem_dealloc(cx.tmem_base, 512);
 }
 
+// tiles != NULL: the caller's tile table (device count *tile_count, at most max_tiles) replaces the per-clip tiles
 int launch(const float* z, const float* codebook, const int64_t* code_offset, int64_t B, int64_t L, int n_codes,
            int64_t* indices, float* zq_bdl, float* zq_rows, unsigned long long* recheck_rows, float* dbg_acc,
-           cudaStream_t stream) {
+           const VqTile* tiles, const int* tile_count, int64_t max_tiles, cudaStream_t stream) {
   static bool attr = false;
   if (!attr) {
-    FDM_CHECK_CUDA(cudaFuncSetAttribute(vq_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    FDM_CHECK_CUDA(cudaFuncSetAttribute(vq_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    FDM_CHECK_CUDA(cudaFuncSetAttribute(vq_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     attr = true;
   }
   Params p;
@@ -955,6 +984,8 @@ int launch(const float* z, const float* codebook, const int64_t* code_offset, in
   FDM_CHECK_ARG(B * ceil_div64(L, TILE_ROWS) < (1ll << 31), "fdm_vq_quantize: too many rows for one launch");
   p.tiles_per_clip = static_cast<int>(ceil_div64(L, TILE_ROWS));
   p.num_tiles = static_cast<int>(B * p.tiles_per_clip);
+  p.tiles = tiles;
+  p.tile_count = tile_count;
   static float wscale = -1.f;
   static bool wscale_set = false;
   if (!wscale_set) {
@@ -967,8 +998,10 @@ int launch(const float* z, const float* codebook, const int64_t* code_offset, in
   static const int l2_ahead = [] { const char* e = getenv("FDM_B200_VQ_L2_AHEAD"); return e ? atoi(e) : L2_AHEAD; }();
   p.l2_ahead = l2_ahead;
   const int64_t sms = fdm_sm_count();
-  const int grid = static_cast<int>(p.num_tiles < sms ? p.num_tiles : sms);
-  vq_tc_kernel<<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(p);
+  const int64_t n_t = tiles ? max_tiles : p.num_tiles;
+  const int grid = static_cast<int>(n_t < sms ? n_t : sms);
+  if (tiles) vq_tc_kernel<true><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(p);
+  else vq_tc_kernel<false><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(p);
   FDM_CHECK_LAUNCH();
   return 0;
 }

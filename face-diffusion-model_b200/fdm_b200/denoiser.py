@@ -21,6 +21,7 @@ import torch
 
 from . import lib
 from .presets import Preset, alibi_slopes
+from .vqvae import check_frame_cond
 
 
 def _sin_table(n: int, d: int) -> torch.Tensor:
@@ -152,7 +153,8 @@ class DenoiserEngine:
     def prepare(self, audio_hidden: torch.Tensor, n_frames: int, id_one_hot: torch.Tensor,
                 emo_one_hot: Optional[torch.Tensor] = None, guidance: Optional[str] = None, fanout: int = 1) -> None:
         """audio_hidden: (A, N, audio_dim) audio-encoder output in the compute dtype; n_frames: latent frames T.
-        fanout: K sequences per audio clip, B = A*K sequences, sequence a*K + k on clip a; the one-hots have B rows or 1.
+        fanout: K sequences per audio clip, B = A*K sequences, sequence a*K + k on clip a; the one-hots have B rows or 1,
+        or are per frame, (B | 1, T, n): frame f of sequence b is conditioned on row [b, f] (any values, e.g. a cross-fade).
         guidance: None, or the name of the condition the unconditional pass zeroes ("id" | "emotion")."""
         self.pack()
         P, w, d = self.P, self.w, self.P.d
@@ -162,7 +164,10 @@ class DenoiserEngine:
         Ta = N // 2 if P.pair_audio else N
         if n_frames > Ta:
             raise ValueError(f"latent has {n_frames} frames but the audio only yields {Ta} (the reference fails here too)")
-        for oh in (id_one_hot, emo_one_hot):  # checked before any buffer changes, so a refused call keeps the prepared state
+        for oh, n in ((id_one_hot, P.n_id), (emo_one_hot, 7)):  # checked before any buffer changes, so a refused call keeps
+            if oh is not None and oh.dim() == 3:                 # the prepared state
+                check_frame_cond(oh, B, n_frames, n)
+                continue
             rows = 1 if oh is None or oh.dim() == 1 else oh.shape[0]
             if rows not in (1, B):
                 raise ValueError(f"a condition has {rows} rows; the call has {B} sequences (give {B} rows or 1)")
@@ -193,13 +198,19 @@ class DenoiserEngine:
                 lib.gemm(h, L["co_w"], cc, bias=L["co_b"])
                 c.view(A, fanout, T, d).copy_(cc.view(A, 1, T, d).expand(A, fanout, T, d))  # setup-time broadcast
             self.cross.append(c)
-        # style (+ emotion) per sequence and pass, plus positional encoding -> one addend tensor per pass
+        # style (+ emotion) per sequence (or per frame) and pass, plus positional encoding -> one addend tensor per pass. With a
+        # per-frame condition both GEMMs run over the B*T frame rows; the FFMA GEMM's rows do not depend on M, so a constant
+        # schedule gives the per-sequence call's bits.
+        per_frame = any(oh is not None and oh.dim() == 3 for oh in (id_one_hot, emo_one_hot))
         def expand(oh, n):
             oh = oh.to(dev, torch.float32)
+            if oh.dim() == 3:
+                return oh.expand(B, T, n).reshape(BT, n).contiguous()
             if oh.dim() == 1:
                 oh = oh[None]
             assert oh.shape[-1] == n
-            return oh.expand(B, n).contiguous() if oh.shape[0] == 1 else oh.contiguous()
+            oh = oh.expand(B, n) if oh.shape[0] == 1 else oh
+            return oh.repeat_interleave(T, dim=0) if per_frame else oh.contiguous()
         ids = expand(id_one_hot, P.n_id)
         emo = expand(emo_one_hot, 7) if P.emotion else None
         passes = [(ids, emo)]
@@ -213,12 +224,12 @@ class DenoiserEngine:
         pe = w["pe"][torch.arange(T, device=dev) % P.period] if P.periodic_pe else _sin_table(T, d).to(dev)
         addends = []
         for (i_oh, e_oh) in passes:
-            sty = torch.empty(B, d, device=dev)
+            sty = torch.empty(i_oh.shape[0], d, device=dev)
             lib.gemm(i_oh, w["st_w"], sty, bias=w["st_b"], act=lib.ACT_MISH if P.style_mish else lib.ACT_NONE)
             if P.emotion:
                 lib.gemm(e_oh, w["em_w"], sty, bias=w["em_b"], residual=sty)
             ad = self.buf(f"addend{len(addends)}", (BT, d), dt)
-            ad.copy_((sty[:, None, :] + pe[None]).reshape(BT, d))  # setup-time broadcast (+ cast)
+            ad.copy_((sty.view(B, -1, d) + pe[None]).reshape(BT, d))  # setup-time broadcast (+ cast)
             addends.append(ad)
         self.addend = addends
         # guidance: both passes share Mish(latent_encoder(x_t)); the second pass is the first plus (addend_1 - addend_0)

@@ -71,6 +71,10 @@ class WindowArgs(C.Structure):
                 ("S", _i64), ("d", _i64)]
 
 
+class VqRuns(C.Structure):
+    _fields_ = [("clip_run", _vp), ("run_l0", _vp), ("run_offset", _vp), ("n_runs", _i64)]
+
+
 EXPORTS = {
     "fdm_last_error": (C.c_char_p, []),
     "fdm_device_info": (C.c_int, [C.POINTER(_i32)] * 3),
@@ -92,6 +96,10 @@ EXPORTS = {
     "fdm_vq_quantize": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _vp]),
     "fdm_vq_quantize_ex": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp, _vp]),
     "fdm_vq_stats": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp, _vp]),
+    "fdm_vq_runs_workspace_bytes": (_i64, [_i64, _i64, _i64]),
+    "fdm_vq_quantize_runs": (C.c_int, [_vp, _vp, C.POINTER(VqRuns), _i64, _i64, _i64, _i64, _vp, _vp, _vp, _i32, _vp, _vp,
+                                       _i64, _vp]),
+    "fdm_vq_stats_runs": (C.c_int, [_vp, _vp, C.POINTER(VqRuns), _vp, _i64, _i64, _i64, _i64, _vp, _i64, _vp, _vp]),
     "fdm_split_bf16x2": (C.c_int, [_vp, _vp, _vp, _i64, _vp]),
     "fdm_cast": (C.c_int, [_vp, _i32, _vp, _i32, _i64, _vp]),
     "fdm_cast_rows": (C.c_int, [_vp, _i64, _vp, _i32, _i64, _i64, _i64, _vp]),
@@ -536,6 +544,49 @@ def vq_quantize(z: torch.Tensor, codebook: torch.Tensor, n_codes: int, code_offs
                                   _ptr(zr), algo, _ptr(recheck_rows), _ptr(dbg_acc), _stream()))
     _launched()
     return idx, zq, zr
+
+
+def _vq_runs(runs, B: int, L: int, device) -> tuple:
+    """(VqRuns, the device tensors it points at) of a run table (clip_run, run_l0, run_offset), int64 host or device tensors."""
+    clip_run, run_l0, run_offset = (torch.as_tensor(t, dtype=torch.int64).to(device).contiguous() for t in runs)
+    assert clip_run.numel() == B + 1 and run_l0.numel() == run_offset.numel() >= B
+    return VqRuns(_ptr(clip_run), _ptr(run_l0), _ptr(run_offset), run_l0.numel()), (clip_run, run_l0, run_offset)
+
+
+def vq_quantize_runs(z: torch.Tensor, codebook: torch.Tensor, n_codes: int, runs, want_bdl=True, want_rows=False,
+                     algo: int = VQ_AUTO, recheck_rows: Optional[torch.Tensor] = None):
+    """vq_quantize with per-row codebook slices: `runs` = (clip_run (B+1), run_l0, run_offset) int64, the CSR run table of
+    fdm_vq_runs (fdm_b200.vqvae.slice_runs builds it). Same outputs and layouts as vq_quantize."""
+    lib = require_device()
+    assert z.dtype == torch.float32 and z.is_contiguous() and codebook.dtype == torch.float32 and codebook.is_contiguous()
+    B, L, D = z.shape
+    rs, keep = _vq_runs(runs, B, L, z.device)
+    idx = torch.empty((B * L, 1), dtype=torch.int64, device=z.device)
+    zq = torch.empty((B, D, L), dtype=torch.float32, device=z.device) if want_bdl else None
+    zr = torch.empty((B, L, D), dtype=torch.float32, device=z.device) if want_rows else None
+    if recheck_rows is not None:
+        assert recheck_rows.dtype == torch.int64 and recheck_rows.numel() == 1
+    n_ws = int(lib.fdm_vq_runs_workspace_bytes(B, L, rs.n_runs))
+    ws = torch.empty((n_ws + 15) // 16 * 4, dtype=torch.int32, device=z.device)
+    _check(lib.fdm_vq_quantize_runs(_ptr(z), _ptr(codebook), C.byref(rs), B, L, D, n_codes, _ptr(idx), _ptr(zq), _ptr(zr),
+                                    algo, _ptr(recheck_rows), _ptr(ws), ws.numel() * 4, _stream()))
+    _launched(2)
+    return idx, zq, zr
+
+
+def vq_stats_runs(z: torch.Tensor, codebook: torch.Tensor, indices: torch.Tensor, n_codes: int, runs):
+    """vq_stats with the slice of every row from a run table (see vq_quantize_runs)."""
+    assert z.dtype == torch.float32 and z.dim() == 3 and z.is_contiguous() and codebook.dtype == torch.float32 and codebook.is_contiguous()
+    assert indices.dtype == torch.int64 and indices.is_contiguous() and indices.numel() == z.shape[0] * z.shape[1]
+    B, L, D = z.shape
+    rs, keep = _vq_runs(runs, B, L, z.device)
+    n_part = int(min(8 * 148, max(1, (B * L + 63) // 64)))
+    partials = torch.empty(n_part, device=z.device, dtype=torch.float32)
+    hist = torch.zeros(n_codes, device=z.device, dtype=torch.int64)
+    _check(require_device().fdm_vq_stats_runs(_ptr(z), _ptr(codebook), C.byref(rs), _ptr(indices), B, L, D, n_codes,
+                                              _ptr(partials), n_part, _ptr(hist), _stream()))
+    _launched()
+    return partials.double().sum(), hist
 
 
 def cast_rows(src: torch.Tensor, dst: torch.Tensor) -> torch.Tensor:

@@ -20,7 +20,7 @@ from .audio import AudioEncoderEngine
 from .denoiser import DenoiserEngine, _sin_table
 from .presets import PRESETS, Preset
 from .sampler import SamplerEngine, pool_known, pool_windows
-from .vqvae import VQDecoderEngine, quantize
+from .vqvae import VQDecoderEngine, check_frame_cond, quantize
 from .windows import WindowPlan, plan_windows
 
 DEFAULT_PRECISION = os.environ.get("FDM_B200_PRECISION", "bf16")
@@ -340,7 +340,9 @@ def cosine_tables(timesteps: int, s: float = 0.008):
 
 class GaussianDiffusionBase(nn.Module):
     """Sampling calls take `audio` (A, L) and a latent of B = A*K sequences: sequence a*K + k uses clip a (the order of
-    audio.repeat_interleave(K, 0)), and each clip's audio work runs once. Condition one-hots have B rows or 1.
+    audio.repeat_interleave(K, 0)), and each clip's audio work runs once. Condition one-hots have B rows or 1, or are per
+    frame: (B | 1, T, n) with T = shape[1] // fq, row [b, f] conditioning frame f of sequence b (rows need not be one-hot: a
+    soft row cross-fades). A 2-D condition is always per sequence. Identity and emotion may be per frame independently.
 
     Known frames (p_sample_loop / sample / ddim_sample): `known` (B or 1, fq*T, zdim) float32, the layout
     VQAutoEncoder.encode returns, and `known_mask` bool (B, T) or (T,), one entry per frame. Masked frames start from
@@ -483,8 +485,11 @@ class GaussianDiffusionBase(nn.Module):
             raise ValueError(f"expected {self.n_cond} condition one-hot(s), got {len(conds)}")
         plan = plan_windows(P, shape, audio.shape[0], audio.shape[1], window, overlap)
         B = plan.A * plan.K
-        for c in conds:
-            if not isinstance(c, torch.Tensor) or c.dim() not in (1, 2) or (c.dim() == 2 and c.shape[0] not in (1, B)):
+        widths = (7, P.n_id) if self.n_cond == 2 else (P.n_id,)
+        for c, n in zip(conds, widths):
+            if isinstance(c, torch.Tensor) and c.dim() == 3:
+                check_frame_cond(c, B, plan.T, n)
+            elif not isinstance(c, torch.Tensor) or c.dim() not in (1, 2) or (c.dim() == 2 and c.shape[0] not in (1, B)):
                 raise ValueError(f"a condition has shape {tuple(getattr(c, 'shape', ()))}; the call has {B} sequences "
                                  f"(give {B} rows or 1)")
         if ddim_steps is not None:
@@ -501,7 +506,7 @@ class GaussianDiffusionBase(nn.Module):
         return plan
 
     def _window_inputs(self, audio: torch.Tensor, idh, emo, plan: WindowPlan):
-        """(window audio, identity rows, emotion rows) of a windowed call (plan.window_audio / plan.repeat_rows), cached on
+        """(window audio, identity rows, emotion rows) of a windowed call (plan.window_audio / plan.window_rows), cached on
         the identity and version of the inputs and the window layout: a repeat call passes the same tensors on, so the
         audio encoder's cache, prepare() and the captured graphs are hit."""
         key = (plan.W, plan.S, plan.n_w, plan.r, plan.K)
@@ -509,7 +514,7 @@ class GaussianDiffusionBase(nn.Module):
         if c is None or c[1] != key or not FDMBase._same(c[0], (audio, idh, emo)):
             with torch.inference_mode(False):  # normal tensors: the caches downstream read their version counters
                 c = (FDMBase._ident((audio, idh, emo)), key,
-                     (plan.window_audio(audio), plan.repeat_rows(idh), plan.repeat_rows(emo)))
+                     (plan.window_audio(audio), plan.window_rows(idh), plan.window_rows(emo)))
             self.__dict__["_long_audio"] = c
         return c[2]
 
@@ -794,19 +799,27 @@ class VQAutoEncoderBase(nn.Module):
     def encode(self, x, one_hot=None):
         """x (B, T, in_dim) motion (template subtracted) -> (B, fq*T, zquant_dim) fp32, the tensor quant() takes
         (reference: models/vq_vae_emotion.py:20-26, models/vq_vae.py:20-26, models/vq_vae_vocaset.py:23-28; for the
-        vocaset / biwi classes the second argument is the unused `x_a`). SURVEY.md section 8(f) item 3."""
+        vocaset / biwi classes the second argument is the unused `x_a`). SURVEY.md section 8(f) item 3.
+        Emotion class: one_hot may be per frame, (B | 1, T, 7); frame f then gets emotion_mapping(one_hot[b, f])."""
+        if self.emotion_sliced and isinstance(one_hot, torch.Tensor) and one_hot.dim() == 3:
+            check_frame_cond(one_hot, x.shape[0], x.shape[1], self.args.n_embed // self.n_local, "the emotion one-hot")
         return self.engine().encode_rows(x, one_hot if self.emotion_sliced else None)
 
     @torch.no_grad()
     def quant(self, x, one_hot=None):
-        """-> (z_q (B, D, L), loss, (perplexity, min_encodings | None, min_encoding_indices (B*L, 1) int64))"""
+        """-> (z_q (B, D, L), loss, (perplexity, min_encodings | None, min_encoding_indices (B*L, 1) int64))
+        Emotion class: one_hot (B | 1, 7) / (7,) picks a codebook slice per clip; (B | 1, T, 7) per frame, T = L // fq: frame f's
+        fq latent rows use slice 256 * argmax(one_hot[b, f]) (first maximum on ties)."""
         if self.emotion_sliced and one_hot is None:
             raise TypeError("quant() of the emotion EVQ-VAE needs the emotion one-hot")
+        fq = self.args.face_quan_num
+        if self.emotion_sliced and one_hot.dim() == 3:
+            check_frame_cond(one_hot, x.shape[0], x.shape[1] // fq, self.args.n_embed // self.n_local, "the emotion one-hot")
         z = x.detach().float().contiguous()
         n_codes = self.n_local if self.emotion_sliced else self.args.n_embed
         with lib.nvtx_range("quantize"):
             idx, zq, zr, sq, hist = quantize(z, self.quantize.embedding.weight, n_codes, one_hot if self.emotion_sliced else None,
-                                             want_bdl=True, want_rows=True, want_stats=True)
+                                             want_bdl=True, want_rows=True, want_stats=True, fq=fq)
         # decode() shortcut: the row layout the quantiser kernel already produced travels WITH the returned tensor
         # (an attribute of that tensor object, valid for its current version), never keyed on an address
         zq._fdm_rows = (zr, zq._version)

@@ -173,10 +173,16 @@ class VQDecoderEngine:
             if emo_one_hot is None:
                 raise TypeError("encode() of the emotion EVQ-VAE needs the emotion one-hot")
             oh = emo_one_hot.to(dev).float()
-            oh = (oh[None] if oh.dim() == 1 else oh).expand(B, -1).contiguous()
-            e = torch.empty(B, d, device=dev, dtype=torch.float32)
-            lib.gemm(oh, w["emo_w"], e, bias=w["emo_b"], act=lib.ACT_LEAKY02)
-            res = e.to(dt).repeat_interleave(T, dim=0)  # emotion_mapping output is added to every frame of its clip
+            if oh.dim() == 3:  # per frame: (B | 1, T, 7), the emotion_mapping output of frame f is added to frame f
+                oh = oh.expand(B, T, -1).reshape(B * T, -1).contiguous()
+                e = torch.empty(B * T, d, device=dev, dtype=torch.float32)
+                lib.gemm(oh, w["emo_w"], e, bias=w["emo_b"], act=lib.ACT_LEAKY02)
+                res = e.to(dt)
+            else:
+                oh = (oh[None] if oh.dim() == 1 else oh).expand(B, -1).contiguous()
+                e = torch.empty(B, d, device=dev, dtype=torch.float32)
+                lib.gemm(oh, w["emo_w"], e, bias=w["emo_b"], act=lib.ACT_LEAKY02)
+                res = e.to(dt).repeat_interleave(T, dim=0)  # emotion_mapping output is added to every frame of its clip
         x = torch.empty(B * T, d, device=dev, dtype=dt)
         lib.gemm(xin, w["vm_w"], x, bias=w["vm_b"], act=lib.ACT_LEAKY02, residual=res)
         k = w["conv_k"]
@@ -217,13 +223,48 @@ class VQDecoderEngine:
         return x
 
 
+def slice_runs(offsets: torch.Tensor, fq: int):
+    """(B, T) int64 codebook offset per frame -> the CSR run table of fdm_vq_runs over the (B, fq*T) latent rows, as host
+    tensors (clip_run (B+1), run_l0, run_offset): a run starts at a clip's first frame and wherever the offset changes."""
+    offsets = offsets.to("cpu", torch.int64)
+    B, T = offsets.shape
+    start = torch.ones(B, T, dtype=torch.bool)
+    start[:, 1:] = offsets[:, 1:] != offsets[:, :-1]
+    b, f = start.nonzero(as_tuple=True)
+    clip_run = torch.zeros(B + 1, dtype=torch.int64)
+    clip_run[1:] = start.sum(1).cumsum(0)
+    return clip_run, f * fq, offsets[b, f].contiguous()
+
+
+def check_frame_cond(oh, B: int, T: int, n: int, what: str = "a condition") -> None:
+    """ValueError unless the per-frame condition `oh` is (B or 1, T, n)."""
+    if oh.shape[0] not in (1, B):
+        raise ValueError(f"{what} has {oh.shape[0]} rows; the call has {B} sequences (give {B} rows or 1)")
+    if oh.shape[1] != T:
+        raise ValueError(f"{what} has {oh.shape[1]} frames; the call has {T} (a per-frame condition is (B | 1, T, n))")
+    if oh.shape[2] != n:
+        raise ValueError(f"{what} has rows of {oh.shape[2]} entries; it needs {n}")
+
+
 def quantize(z: torch.Tensor, codebook: torch.Tensor, n_local: int, emo_one_hot: Optional[torch.Tensor] = None,
-             want_bdl: bool = True, want_rows: bool = False, want_stats: bool = False):
+             want_bdl: bool = True, want_rows: bool = False, want_stats: bool = False, fq: int = 1):
     """z (B, L, D) fp32. Per-clip emotion slice: offset = n_local * argmax(one_hot[b]) (the reference takes a
-    global argmax because it only ever sees B = 1, models/vq_vae_emotion.py:223). want_stats: also the by-products of the
-    reference forward (sum of squared quantisation errors as a 0-d fp64 tensor, code histogram) from one more pass over z."""
+    global argmax because it only ever sees B = 1, models/vq_vae_emotion.py:223). A per-frame one-hot (B | 1, L / fq, n)
+    gives frame f's fq latent rows the slice n_local * argmax(one_hot[b, f]) (fdm_vq_quantize_runs). want_stats: also the
+    by-products of the reference forward (sum of squared quantisation errors as a 0-d fp64 tensor, code histogram) from one
+    more pass over z."""
     z = z.contiguous().float()
     B = z.shape[0]
+    if emo_one_hot is not None and emo_one_hot.dim() == 3:
+        T = z.shape[1] // fq
+        pos = torch.argmax(emo_one_hot, dim=-1).to(torch.int64).expand(B, T)
+        runs = slice_runs(pos * n_local, fq)
+        cb = codebook.detach().float().contiguous()
+        idx, zq, zr = lib.vq_quantize_runs(z, cb, n_local, runs, want_bdl=want_bdl, want_rows=want_rows)
+        if want_stats:
+            sq, hist = lib.vq_stats_runs(z, cb, idx.view(-1), n_local, runs)
+            return idx, zq, zr, sq, hist
+        return idx, zq, zr
     off = None
     if emo_one_hot is not None:
         oh = emo_one_hot.to(z.device)

@@ -85,6 +85,20 @@ class WindowPlan:
         n = cond.shape[-1]
         return cond.reshape(self.A, 1, self.K, n).expand(self.A, self.n_w, self.K, n).reshape(self.n_seq, n)
 
+    def gather_frames(self, cond: torch.Tensor) -> torch.Tensor:
+        """A per-frame condition (A*K or 1, T, n) -> (A*n_w*K, W, n): window w's rows are frames [w*S, w*S + W), frames at
+        or past T (sampled on zero audio and dropped) take frame T - 1's row."""
+        n = cond.shape[-1]
+        f = self.frame_index().clamp(max=self.T - 1).to(cond.device)
+        x = cond.expand(self.A * self.K, self.T, n).reshape(self.A, self.K, self.T, n)[:, :, f]  # (A, K, n_w, W, n)
+        return x.permute(0, 2, 1, 3, 4).reshape(self.n_seq, self.W, n).contiguous()
+
+    def window_rows(self, cond: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+        """The condition of the window sequences: gather_frames for a per-frame (3-D) condition, else repeat_rows."""
+        if cond is not None and cond.dim() == 3:
+            return self.gather_frames(cond)
+        return self.repeat_rows(cond)
+
     def frame_index(self) -> torch.Tensor:
         """(n_w, W) absolute frame of every window row."""
         return torch.arange(self.n_w)[:, None] * self.S + torch.arange(self.W)[None, :]

@@ -290,6 +290,31 @@ int fdm_vq_stats(const float* z, const float* codebook, const int64_t* code_offs
                  int64_t L, int64_t D, int64_t n_codes, float* sqerr_partials, int64_t n_partials, int64_t* hist,
                  void* stream);
 
+/* Per-row codebook slices (per-frame emotion schedules), as a run table in CSR form: the rows of clip b are cut into runs
+ * clip_run[b] .. clip_run[b + 1] - 1 (clip_run[0] = 0, clip_run[B] = n_runs); run r covers rows [run_l0[r], next run's
+ * run_l0, or L) of its clip and uses the slice [run_offset[r], run_offset[r] + n_codes). A clip's first run starts at row 0
+ * and run_l0 ascends within a clip. Device arrays, written before the call. One run per clip is fdm_vq_quantize_ex with
+ * code_offset[b] = run_offset[b], bit for bit. */
+typedef struct fdm_vq_runs {
+  const int64_t* clip_run;    /* [B + 1] */
+  const int64_t* run_l0;      /* [n_runs] */
+  const int64_t* run_offset;  /* [n_runs] */
+  int64_t n_runs;
+} fdm_vq_runs;
+/* Bytes of the caller-owned device workspace of fdm_vq_quantize_runs (its tile table: no tile crosses a run). */
+int64_t fdm_vq_runs_workspace_bytes(int64_t B, int64_t L, int64_t n_runs);
+/* fdm_vq_quantize_ex with the run table instead of code_offset: same expression, same outputs and layouts, same algo
+ * selection. The call first cuts the runs into tiles of the chosen kernel (a small one-CTA kernel writes the table into
+ * `workspace`, 16-byte aligned, at least fdm_vq_runs_workspace_bytes), then quantises tile by tile; a run's last tile
+ * may be partial. */
+int fdm_vq_quantize_runs(const float* z, const float* codebook, const fdm_vq_runs* runs, int64_t B, int64_t L, int64_t D,
+                         int64_t n_codes, int64_t* indices, float* zq_bdl, float* zq_rows, int32_t algo,
+                         uint64_t* recheck_rows, void* workspace, int64_t workspace_bytes, void* stream);
+/* fdm_vq_stats with the slice of every row taken from the run table. */
+int fdm_vq_stats_runs(const float* z, const float* codebook, const fdm_vq_runs* runs, const int64_t* indices, int64_t B,
+                      int64_t L, int64_t D, int64_t n_codes, float* sqerr_partials, int64_t n_partials, int64_t* hist,
+                      void* stream);
+
 /* ---- small data-movement kernels ------------------------------------------------------------ */
 /* hi = bf16(x), lo = bf16(x - hi): the operand pair of the split-bf16 GEMM (fdm_gemm_args.A_lo / W_lo). n elements. */
 int fdm_split_bf16x2(const float* src, void* hi, void* lo, int64_t n, void* stream);
